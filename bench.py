@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the hybrid-MPC hot path (contract: see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scenarios S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scenarios S] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): the per-vehicle local MIQPs of fleet_decent_mld.py /
 fleet_seq_mld.py at n = 10 vehicles, horizon N = 6, pwa_gear model.  One STEP = one pass of the
@@ -38,6 +38,25 @@ def make_batch(seed, scenarios):
     from hybrid_vehicle_platoon_b200.synth_local import platoon_local_problems
     rng = np.random.default_rng(seed)
     return platoon_local_problems(rng, scenarios, N_VEH, HORIZON)
+
+
+def dump_outputs(out_dir, arrays, limit_bytes=64_000_000, seed=0):
+    """Writes `arrays` (name -> CUDA tensor, first axis = problem) as <out_dir>/<name>.npy in float64, so that two builds
+    can be compared output for output.  When they would exceed `limit_bytes` in all, every array keeps the same seeded
+    sample of problems (in index order) and the sampled problem indices go to sample_index.npy."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    first = next(iter(arrays.values()))
+    B = first.shape[0]
+    row_bytes = 8 * sum(a[0].numel() for a in arrays.values())
+    if B * row_bytes > limit_bytes:
+        k = (limit_bytes - 4096) // (row_bytes + 8)          # 8 B per problem for the index; 4 KiB for the headers
+        idx = np.sort(np.random.default_rng(seed).choice(B, k, replace=False))
+        sel = torch.from_numpy(idx).to(first.device)
+        arrays = {n: a.index_select(0, sel) for n, a in arrays.items()}
+        np.save(os.path.join(out_dir, "sample_index.npy"), idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.cpu().numpy().astype(np.float64))
 
 
 def peaks():
@@ -416,7 +435,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--profile", action="store_true",
                     help="short run for ncu: device-timed MIQP steps + rollout launches only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the solutions of the last timed step (u, x, modes, obj, status; rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -487,6 +512,9 @@ def main():
     ms = np.array([a.elapsed_time(b_) for a, b_ in ev])
     total_ms = float(ms.sum())
     assert bool((d_status == 2).all()), "a bench problem was not solved to optimality"
+    if args.dump_outputs and rank == 0:
+        # node and QP-iteration counts are left out: which worker adopts which sub-tree depends on scheduling
+        dump_outputs(args.dump_outputs, {"u": d_u, "x": d_x, "modes": d_modes, "obj": d_obj, "status": d_status})
     nodes_mean = float(d_nodes.double().mean())
     iters_mean = float(d_iters.double().mean())
 

@@ -264,24 +264,21 @@ def use_all_cores() -> int:
 _BNB = {}
 
 
-def _cpu_tag() -> str:
-    """Identifies the host CPU, so that a -march=native build made on another machine is never loaded."""
-    import hashlib
-    try:
-        with open("/proc/cpuinfo") as f:
-            txt = f.read()
-        keep = [ln for ln in txt.splitlines() if ln.startswith(("model name", "flags"))][:2]
-        return hashlib.sha1("\n".join(keep).encode()).hexdigest()[:12]
-    except OSError:
-        return "unknown"
-
-
 def build_cpu_bnb(native: bool = False, force: bool = False) -> str:
-    """Generic build: libhvp_cpu_bnb.so (-O3).  Native build: libhvp_cpu_bnb_native_<cpu tag>.so (-O3 -march=native),
-    compiled on the machine that runs it (a native build does not travel between hosts)."""
+    """Generic build: oracle/libhvp_cpu_bnb.so (-O3).  Native build (-O3 -march=native): compiled by the process that
+    loads it into a temporary directory removed at exit, so it never travels between hosts and the tree may be
+    read-only."""
     src = os.path.join(_HERE, "hvp_cpu_bnb.cpp")
     hdr = os.path.join(_HERE, "..", "hybrid_vehicle_platoon_b200", "csrc", "flat_core.cuh")
-    out = os.path.join(_HERE, f"libhvp_cpu_bnb_native_{_cpu_tag()}.so" if native else "libhvp_cpu_bnb.so")
+    if native:
+        import atexit
+        import shutil
+        import tempfile
+        tmp = tempfile.mkdtemp(prefix="hvp_cpu_bnb_")
+        atexit.register(shutil.rmtree, tmp, ignore_errors=True)
+        out = os.path.join(tmp, "libhvp_cpu_bnb_native.so")
+    else:
+        out = os.path.join(_HERE, "libhvp_cpu_bnb.so")
     newest = max(os.path.getmtime(src), os.path.getmtime(hdr))
     if force or not os.path.exists(out) or os.path.getmtime(out) < newest:
         cxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"

@@ -35,6 +35,34 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert p.returncode == 0 and p.stdout.strip() == ""
 
 
+def test_dump_outputs_writes_float64_and_one_shared_sample_above_the_limit(tmp_path):
+    """bench.dump_outputs (--dump-outputs): every array whole while they fit, else the same seeded problems of each
+    array (indices in sample_index.npy), within the byte limit and identical from call to call."""
+    import importlib
+    import numpy as np
+    import torch
+    bench = importlib.import_module("bench")
+    B = 1000
+    arrays = {"obj": torch.arange(B, dtype=torch.float64), "u": torch.arange(B * 6, dtype=torch.float64).reshape(B, 6),
+              "status": torch.full((B,), 2, dtype=torch.int32)}
+    bench.dump_outputs(str(tmp_path / "all"), arrays)
+    assert sorted(p.name for p in (tmp_path / "all").iterdir()) == ["obj.npy", "status.npy", "u.npy"]
+    for name, a in arrays.items():
+        d = np.load(tmp_path / "all" / f"{name}.npy")
+        assert d.dtype == np.float64 and np.array_equal(d, a.numpy())
+    limit = 40_000
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays, limit_bytes=limit)
+    files = sorted((tmp_path / "a").iterdir())
+    assert sum(p.stat().st_size for p in files) <= limit
+    idx = np.load(tmp_path / "a" / "sample_index.npy").astype(np.int64)
+    assert 0 < len(idx) < B and (np.diff(idx) > 0).all()
+    assert np.array_equal(np.load(tmp_path / "a" / "obj.npy"), idx) and (np.load(tmp_path / "a" / "status.npy") == 2).all()
+    assert np.array_equal(np.load(tmp_path / "a" / "u.npy"), arrays["u"].numpy()[idx])
+    for p in files:
+        assert np.array_equal(np.load(p), np.load(tmp_path / "b" / p.name))
+
+
 def test_episode_legs_warm_up_at_full_size_and_report_the_median():
     """bench._episodes: one untimed run first (idle clocks, cold allocator), then the median of the timed runs, each
     bracketed by the caller's sync and reduced over the ranks by the caller's reduction."""

@@ -2,8 +2,8 @@
 SURVEY.md 8c: the MIQP half of the path is "parity unpinned" in this container (no Gurobi, no dmpcpwa, no
 network); this test closes the pin automatically on a box that has them:
     HVP_REFERENCE_DIR=/path/to/hybrid-vehicle-platoon python -m pytest tests/test_live_gurobi.py -m gpu
-It is skipped (importorskip) everywhere else -- including the GPU box of this build, where /root/reference
-does not exist.  Tolerances are BASELINE.json's: objective 1e-6 relative, inputs 1e-5."""
+It is skipped everywhere else: without gurobipy, without dmpcpwa, or without HVP_REFERENCE_DIR naming a checkout of
+the reference.  Tolerances are BASELINE.json's: objective 1e-6 relative, inputs 1e-5."""
 import os
 import sys
 
@@ -12,15 +12,15 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 
-REF = os.environ.get("HVP_REFERENCE_DIR", "/root/reference")
+REF = os.environ.get("HVP_REFERENCE_DIR")
 
 
 @pytest.fixture(scope="module")
 def ref():
     pytest.importorskip("gurobipy")
     pytest.importorskip("dmpcpwa")
-    if not os.path.isdir(REF):
-        pytest.skip(f"reference sources not found at {REF}")
+    if not REF or not os.path.isdir(REF):
+        pytest.skip("HVP_REFERENCE_DIR does not name a checkout of the reference sources")
     sys.path.insert(0, REF)
     import fleet_decent_mld as ref_decent        # the reference's own module
     import models as ref_models
