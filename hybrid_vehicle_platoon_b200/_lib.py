@@ -63,6 +63,15 @@ class AdmmRound(C.Structure):      # hvp_admm_round
                [(k, C.c_void_p) for k in ("lwin", "y_front", "y_back", "zf", "zb", "xs")]
 
 
+class CentStep(C.Structure):       # hvp_cent_step
+    _fields_ = [("n", C.c_int32), ("N", C.c_int32), ("S", C.c_int32), ("phase", C.c_int32), ("n_param", C.c_int32),
+                ("leader_per_scenario", C.c_int32), ("leader_len", C.c_int64), ("T", C.c_int64), ("n_modes", C.c_int32),
+                ("reserved", C.c_int32), ("mode_gear", C.c_int32 * 16)] + \
+               [(k, C.c_void_p) for k in ("t", "leader_x", "params", "u", "modes", "obj", "status", "nodes", "u0", "gear0",
+                                          "U_log", "obj_log", "status_log", "nodes_log", "aborted_at")]
+
+
+CENT_PACK, CENT_ADOPT = 0, 1
 MPC_CENT, MPC_LOCAL, MPC_EVENT, MPC_ADMM, MPC_GADMM = 1, 2, 3, 4, 5
 MODEL_PWA_GEAR, MODEL_FRICTION_GEAR = 0, 1
 REAL_VEHICLE_REF, NO_LEADER = 8, -100
@@ -123,6 +132,7 @@ def lib():
     L.hvp_gadmm_round_dev.argtypes = [_vp, C.POINTER(GAdmmRound), _vp]
     L.hvp_decent_observe_dev.argtypes = [_vp, C.POINTER(DecentObserve), _vp]
     L.hvp_admm_round_dev.argtypes = [_vp, C.POINTER(AdmmRound), _vp]
+    L.hvp_cent_step_dev.argtypes = [_vp, C.POINTER(CentStep), _vp]
     L.hvp_microbench_fp64.argtypes = [_vp, C.c_int, C.POINTER(C.c_double)]
     L.hvp_microbench_smem.argtypes = [_vp, C.c_int, C.POINTER(C.c_double)]
     _lib = L

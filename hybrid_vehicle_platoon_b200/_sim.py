@@ -37,7 +37,12 @@ def collect(env, agent, leader_x, fname: str, save: bool, node_counts=None):
                node_counts=agent.node_counts if node_counts is None else node_counts,
                violations=env.unwrapped.viol_counter[-1], leader_x=leader_x)
     if save:
-        with open(fname, "wb") as f:
-            for k in ("X", "U", "R", "solve_times", "node_counts", "violations", "leader_x"):
-                pickle.dump(out[k], f)
+        save_results(out, fname)
     return out
+
+
+def save_results(out: dict, fname: str) -> None:
+    """The reference's pickle: the 7 result objects dumped one after the other, in this order."""
+    with open(fname, "wb") as f:
+        for k in ("X", "U", "R", "solve_times", "node_counts", "violations", "leader_x"):
+            pickle.dump(out[k], f)

@@ -230,3 +230,11 @@ def admm_round_device(g, *, pack_only: bool = False, ctx=None, stream=None):
     ctx = ctx or default_context()
     g.pack_only = 1 if pack_only else 0
     check(lib().hvp_admm_round_dev(ctx.handle, C.byref(g), _stream_arg(stream)))
+
+
+def cent_step_device(g, *, phase: int, ctx=None, stream=None):
+    """Fused glue of a centralized timestep (hvp_cent_step_dev): phase _lib.CENT_PACK writes the leader window into the
+    parameter rows, _lib.CENT_ADOPT adopts the solve's answer and logs it; `g` is a _lib.CentStep."""
+    ctx = ctx or default_context()
+    g.phase = int(phase)
+    check(lib().hvp_cent_step_dev(ctx.handle, C.byref(g), _stream_arg(stream)))

@@ -290,6 +290,66 @@ admm_round_kernel(const __grid_constant__ AdmmArgs A) {
     }
 }
 
+// ---- centralized controller: the leader window before the solve, the adoption of its answer after it
+// (fleet_cent_mld.py:22-32, mpcs/mpc_gear.py:116-135) -------------------------------------------------------------
+struct CentArgs {
+    int n, N, S, phase, npar, n_modes;
+    long long lx_len, lx_sstride, T;  // leader trajectory: [S or 1][2][lx_len], scenario stride 0 when shared
+    int mode_gear[16];
+    const long long* t;
+    const double* lx;
+    double* params;
+    const double *u, *obj;
+    const int32_t *modes, *status, *nodes;
+    double* u0;
+    int32_t* gear0;
+    double *U, *objl;
+    int32_t *stl, *ndl, *ab;
+};
+__global__ void __launch_bounds__(128)
+cent_step_kernel(const __grid_constant__ CentArgs A) {
+    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = A.n, N = A.N, np1 = N + 1;
+    if (tid >= (int64_t)A.S * n) return;
+    const int s = (int)(tid / n), i = (int)(tid - (int64_t)s * n);
+    const long long t = *A.t;
+    if (A.phase == HVP_CENT_PACK) {
+        // the scenario's n threads share the 2(N+1) entries of the window
+        const double* l = A.lx + (size_t)s * A.lx_sstride;
+        double* P = A.params + (size_t)s * A.npar;
+        for (int e = i; e < 2 * np1; e += n) {
+            const int row = e / np1, k = e - row * np1;
+            long long c = t + k;
+            c = c < 0 ? 0 : (c >= A.lx_len ? A.lx_len - 1 : c);
+            P[e] = l[row * A.lx_len + c];
+        }
+        return;
+    }
+    const bool ok = A.status[s] == HVP_OPTIMAL;
+    const double u0 = ok ? A.u[(size_t)tid * N] : 0.0;
+    A.u0[tid] = u0;
+    int gear = 6;
+    if (A.gear0) {
+        if (ok) {
+            int m = A.modes[(size_t)tid * N];
+            m = m < 0 ? 0 : (m >= A.n_modes ? A.n_modes - 1 : m);
+            gear = A.mode_gear[m];
+        }
+        A.gear0[tid] = gear;
+    }
+    if (t < 0 || t >= A.T) return;
+    const int w = A.gear0 ? 2 * n : n;
+    double* Ur = A.U + ((size_t)t * A.S + s) * w;
+    Ur[i] = u0;
+    if (A.gear0) Ur[n + i] = (double)gear;
+    if (i == 0) {
+        const size_t r = (size_t)t * A.S + s;
+        A.objl[r] = A.obj[s]; A.stl[r] = A.status[s]; A.ndl[r] = A.nodes[s];
+        if (t == 0) A.ab[s] = ok ? -1 : 0;
+        else if (!ok && A.ab[s] < 0) A.ab[s] = (int32_t)t;
+    }
+}
+
 }  // namespace hvp
 
 using namespace hvp;
@@ -391,6 +451,44 @@ extern "C" int hvp_admm_round_dev(hvp_ctx* c, const hvp_admm_round* g, void* str
     admm_round_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(A);
     e = cudaGetLastError();
     if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "admm_round: launch failed: %s", cudaGetErrorString(e));
+    c->launches += 1;
+    return 0;
+}
+
+// hvp.h: hvp_cent_step_dev
+extern "C" int hvp_cent_step_dev(hvp_ctx* c, const hvp_cent_step* g, void* stream) {
+    if (!c || !g) return hvp_fail(-1, "cent_step: NULL argument");
+    if (g->n < 1 || g->N < 1 || g->S < 0 ||
+        (g->phase != HVP_CENT_PACK && g->phase != HVP_CENT_ADOPT))
+        return hvp_fail(-4, "cent_step: bad sizes (n=%d N=%d S=%d phase=%d)", g->n, g->N, g->S, g->phase);
+    CentArgs A;
+    A.n = g->n; A.N = g->N; A.S = g->S; A.phase = g->phase; A.npar = g->n_param; A.n_modes = g->n_modes;
+    A.lx_len = g->leader_len; A.lx_sstride = g->leader_per_scenario ? 2 * g->leader_len : 0; A.T = g->T;
+    A.t = (const long long*)g->t; A.lx = g->leader_x; A.params = g->params;
+    A.u = g->u; A.obj = g->obj; A.modes = g->modes; A.status = g->status; A.nodes = g->nodes;
+    A.u0 = g->u0; A.gear0 = g->gear0; A.U = g->U_log; A.objl = g->obj_log; A.stl = g->status_log; A.ndl = g->nodes_log;
+    A.ab = g->aborted_at;
+    if (g->phase == HVP_CENT_PACK) {
+        if (g->n_param < 2 * (g->N + 1) || g->leader_len < 1)
+            return hvp_fail(-4, "cent_step: bad sizes (n_param=%d leader_len=%lld, N=%d)", g->n_param, (long long)g->leader_len, g->N);
+        if (g->S == 0) return 0;
+        if (!g->t || !g->leader_x || !g->params) return hvp_fail(-1, "cent_step: NULL array argument (pack)");
+    } else {
+        if (g->T < 0 || (g->gear0 && (g->n_modes < 1 || g->n_modes > 16)))
+            return hvp_fail(-4, "cent_step: bad sizes (T=%lld n_modes=%d)", (long long)g->T, g->n_modes);
+        if (g->S == 0) return 0;
+        if (!g->t || !g->u || !g->obj || !g->status || !g->nodes || !g->u0 || !g->U_log || !g->obj_log || !g->status_log ||
+            !g->nodes_log || !g->aborted_at || (g->gear0 && !g->modes))
+            return hvp_fail(-1, "cent_step: NULL array argument (adopt)");
+        for (int m = 0; m < 16; ++m) A.mode_gear[m] = g->mode_gear[m];
+    }
+    cudaError_t e = cudaSetDevice(c->device);
+    if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "cent_step: cudaSetDevice: %s", cudaGetErrorString(e));
+    cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
+    const int64_t threads = (int64_t)g->S * g->n;
+    cent_step_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(A);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "cent_step: launch failed: %s", cudaGetErrorString(e));
     c->launches += 1;
     return 0;
 }

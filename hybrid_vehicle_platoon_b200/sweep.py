@@ -1230,3 +1230,134 @@ class BatchedEventSweep:
         torch.cuda.synchronize()
         return dict(X=X.cpu().numpy(), U=U.cpu().numpy(), R=R.cpu().numpy(), violations=V.cpu().numpy(),
                     errors=E.cpu().numpy(), winners=WIN.cpu().numpy(), feasible=FEAS.cpu().numpy(), nodes=ND.cpu().numpy())
+
+
+class BatchedCentSweep:
+    """S independent platoons under the centralized MLD-MPC (TrackingCentralizedAgent with MpcMldCent / MpcGearCent,
+    fleet_cent_mld.py:14-101), all state on the device.  One timestep, for all S scenarios: pack the leader window
+    leader_x[:, t:t+N+1] into every parameter row, ONE compiled-MPC launch of S centralized problems, adopt the answers
+    (inputs, gears from the mode table, logs) -- pack and adopt are the two phases of hvp_cent_step_dev
+    (csrc/coord.cu) -- ONE rollout launch, and the X / R / violation / error logs at the device-side timestep index
+    (no host synchronisation and no host copy until the results are read back).
+    Either cost norm (quadratic_cost) and either vehicle model: "pwa_gear" (gears derived from the velocities) or
+    "pwa_friction" (discrete gears chosen by the MPC; the action is [u_g ; gears])."""
+
+    def __init__(self, n: int, N: int, masses=None, spacing_policy=ConstantSpacingPolicy(50), leader_index: int = 0,
+                 quadratic_cost: bool = True, model: str = "pwa_gear", d_safe: float = Params.d_safe,
+                 mip_gap: float = 0.0, time_limit_ms: float = 0.0, device: int = 0, ctx=None):
+        import torch
+        from ._lib import MODEL_FRICTION_GEAR, MODEL_PWA_GEAR, MPC_CENT
+        if model not in ("pwa_gear", "pwa_friction"):
+            raise ValueError(f"model must be 'pwa_gear' or 'pwa_friction', got {model!r}")
+        if n < 1 or N < 1 or n * N > 64:
+            raise ValueError(f"the centralized problem needs 1 <= n * N <= 64 (n = {n}, N = {N})")
+        if not 0 <= leader_index < n:
+            raise ValueError(f"leader_index {leader_index} out of range for n = {n}")
+        self.torch, self.n, self.N, self.leader_index = torch, n, N, leader_index
+        self.quadratic, self.friction = bool(quadratic_cost), model == "pwa_friction"
+        self.dev = torch.device("cuda", device)
+        self.ctx = ctx or default_context(device)
+        self.d0, self.t0 = spacing_params(spacing_policy)
+        self.d_safe = d_safe
+        self.masses = None if masses is None else np.asarray(masses, dtype=np.float64)   # (n,) or (S,n)
+        self.cm = api.CompiledMpc(MPC_CENT, N, n_local=n, model=MODEL_FRICTION_GEAR if self.friction else MODEL_PWA_GEAR,
+                                  leader_index=leader_index, d0=self.d0, t0=self.t0, one_norm=not self.quadratic,
+                                  mip_gap=mip_gap, time_limit_ms=time_limit_ms, ctx=self.ctx)
+
+    def close(self):
+        """Releases the compiled formulation (its device scratch)."""
+        if self.cm is not None:
+            self.cm.close()
+            self.cm = None
+
+    def run(self, x0, leader_x, ep_len: int, strict: bool = False):
+        """x0 (S,2n) initial states, leader_x (2,>=ep_len+N+1) shared or (S,2,>=ep_len+N+1) per scenario.  Returns dict
+        of numpy arrays: X (T+1,S,2n), U (T,S,n) -- (T,S,2n) = [u_g ; gears] for pwa_friction --, R (T,S), violations
+        (T,S) uint8, errors (T,S) int32, obj (T,S), status (T,S) int32, nodes (T,S) int32 and aborted_at (S,) int32 (the
+        first timestep whose solve was not optimal, -1: none).  A non-optimal solve applies zero inputs (gear 6), as
+        solve_mpc(raises=False) does; strict=True raises RuntimeError after the run if there was one."""
+        from . import _lib
+        torch, dev, n, N, cm = self.torch, self.dev, self.n, self.N, self.cm
+        f64, i32 = torch.float64, torch.int32
+        if cm is None:
+            raise RuntimeError("BatchedCentSweep is closed")
+        x0 = np.ascontiguousarray(x0, dtype=np.float64)
+        if x0.ndim != 2 or x0.shape[1] != 2 * n:
+            raise ValueError(f"x0 must have shape (S, {2 * n}), got {x0.shape}")
+        S, T = x0.shape[0], int(ep_len)
+        lx_np = np.ascontiguousarray(leader_x, dtype=np.float64)
+        if lx_np.ndim not in (2, 3) or lx_np.shape[-2] != 2 or (lx_np.ndim == 3 and lx_np.shape[0] != S):
+            raise ValueError(f"leader_x must have shape (2, L) or ({S}, 2, L), got {lx_np.shape}")
+        if lx_np.shape[-1] < T + N + 1:
+            raise ValueError("leader trajectory shorter than ep_len + N + 1")
+        x = torch.as_tensor(x0, device=dev)
+        lx = torch.as_tensor(lx_np, device=dev)
+        m = np.full((S, n), 800.0) if self.masses is None else np.broadcast_to(self.masses, (S, n))
+        d_mass = torch.as_tensor(np.array(m, dtype=np.float64, order="C"), device=dev)
+        edesc = api.env_desc(n, self.leader_index, self.d0, self.t0, self.d_safe, self.quadratic, False, True)
+        w = 2 * n if self.friction else n
+        # solve buffers and the rollout's inputs, allocated once per run
+        params = torch.zeros((S, cm.n_param), dtype=f64, device=dev)
+        uo = torch.empty((S, n, N), dtype=f64, device=dev); xo = torch.empty((S, n, 2, N + 1), dtype=f64, device=dev)
+        mo = torch.empty((S, n, N), dtype=i32, device=dev); ob = torch.empty(S, dtype=f64, device=dev)
+        st = torch.empty(S, dtype=i32, device=dev); no = torch.empty(S, dtype=i32, device=dev)
+        u0 = torch.empty((S, n), dtype=f64, device=dev)
+        gear0 = torch.empty((S, n), dtype=i32, device=dev) if self.friction else None
+        lead_t = torch.empty((S, 2), dtype=f64, device=dev)
+        x_cur = x.clone(); x_next = torch.empty_like(x_cur)
+        r_t = torch.empty(S, dtype=f64, device=dev); v_t = torch.empty(S, dtype=torch.uint8, device=dev)
+        e_t = torch.empty(S, dtype=i32, device=dev)
+        t_idx = torch.zeros(1, dtype=torch.int64, device=dev)
+        # episode logs
+        X = torch.empty((T + 1, S, 2 * n), dtype=f64, device=dev)
+        U = torch.empty((T, S, w), dtype=f64, device=dev)
+        R = torch.empty((T, S), dtype=f64, device=dev)
+        V = torch.empty((T, S), dtype=torch.uint8, device=dev)
+        E = torch.empty((T, S), dtype=i32, device=dev)
+        OBJ = torch.empty((T, S), dtype=f64, device=dev)
+        ST = torch.empty((T, S), dtype=i32, device=dev)
+        ND = torch.empty((T, S), dtype=i32, device=dev)
+        AB = torch.full((S,), -1, dtype=i32, device=dev)
+        X[0] = x
+
+        g = _lib.CentStep()
+        g.n, g.N, g.S, g.n_param = n, N, S, cm.n_param
+        g.leader_per_scenario, g.leader_len, g.T = int(lx.ndim == 3), lx.shape[-1], T
+        g.n_modes = cm.n_modes
+        for k, gear in enumerate(cm.mode_gear.tolist()):
+            g.mode_gear[k] = gear
+        ptr = lambda t_: None if t_ is None else t_.data_ptr()
+        g.t, g.leader_x, g.params = t_idx.data_ptr(), lx.data_ptr(), params.data_ptr()
+        g.u, g.modes, g.obj, g.status, g.nodes = uo.data_ptr(), mo.data_ptr(), ob.data_ptr(), st.data_ptr(), no.data_ptr()
+        g.u0, g.gear0 = u0.data_ptr(), ptr(gear0)
+        g.U_log, g.obj_log, g.status_log, g.nodes_log, g.aborted_at = (t_.data_ptr() for t_ in (U, OBJ, ST, ND, AB))
+
+        def body():
+            stream = torch.cuda.current_stream().cuda_stream
+            api.cent_step_device(g, phase=_lib.CENT_PACK, ctx=self.ctx, stream=stream)        # leader_x[:, t:t+N+1]
+            # x_cur (S, 2n) = [p0 v0 p1 v1 ...] is already the solve's x0 layout [S][n][2]
+            cm.solve_device(S, x_cur, d_mass, params, None, uo, xo, None, mo, ob, st, no, None, stream=stream)
+            api.cent_step_device(g, phase=_lib.CENT_ADOPT, ctx=self.ctx, stream=stream)
+            lead_t.copy_(lx.index_select(-1, t_idx).squeeze(-1))                             # leader_x[:, t]
+            api.rollout_step_device(edesc, S, x_cur, u0, gear0, d_mass, lead_t, x_next, r_t, v_t, e_t, ctx=self.ctx,
+                                    stream=stream)
+            X.index_copy_(0, t_idx + 1, x_next.unsqueeze(0))
+            R.index_copy_(0, t_idx, r_t.unsqueeze(0))
+            V.index_copy_(0, t_idx, v_t.unsqueeze(0)); E.index_copy_(0, t_idx, e_t.unsqueeze(0))
+            x_cur.copy_(x_next)
+            t_idx.add_(1)
+
+        # Eager launches: replaying a timestep as a CUDA graph was measured no faster at any batch size (0.99-1.02x at
+        # S = 10 .. 4096, DESIGN.md 5b) -- the loop is bound by the solve, not by launches
+        for _ in range(T):
+            body()
+        torch.cuda.synchronize()
+        out = dict(X=X.cpu().numpy(), U=U.cpu().numpy(), R=R.cpu().numpy(), violations=V.cpu().numpy(),
+                   errors=E.cpu().numpy(), obj=OBJ.cpu().numpy(), status=ST.cpu().numpy(), nodes=ND.cpu().numpy(),
+                   aborted_at=AB.cpu().numpy())
+        if strict and (out["status"] != _lib.OPTIMAL).any():
+            # raised after the run: nothing can be raised from inside a captured timestep
+            ts_, ss_ = np.nonzero(out["status"] != _lib.OPTIMAL)
+            bad = [f"scenario {s} at timestep {t} (status {out['status'][t, s]})" for t, s in zip(ts_[:8], ss_[:8])]
+            raise RuntimeError(f"Infeasible problem encountered: {', '.join(bad)}{' ...' if len(ts_) > 8 else ''}")
+        return out

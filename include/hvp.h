@@ -309,6 +309,42 @@ typedef struct {
 } hvp_admm_round;
 int hvp_admm_round_dev(hvp_ctx* ctx, const hvp_admm_round* g, void* stream);
 
+/* ---- fused glue of a centralized timestep ---------------------------------------------------------------------
+ * What TrackingCentralizedAgent (fleet_cent_mld.py:22-32) and MpcMldCent / MpcGearCent.solve_mpc (mpcs/mpc_gear.py:
+ * 116-135) do around the solve, for all S scenarios at once, one thread per (scenario, vehicle).  t is read from DEVICE
+ * memory so that a timestep can be replayed as a CUDA graph.  Two phases:
+ *   HVP_CENT_PACK  (before hvp_mpc_solve_dev of the CENT handle): params[s][0 : 2(N+1)] = leader_x[:, t : t+N+1], the
+ *       CENT parameter block 0 ([p_t..p_t+N, v_t..v_t+N]); the rest of each params row is left alone.  leader_x is
+ *       [2][leader_len] shared or [S][2][leader_len].  No column outside [0, leader_len) is ever read: a column index
+ *       t + k past the end reads the last column leader_x[:, leader_len - 1] instead (a caller that wants the
+ *       reference's window checks leader_len >= t + N + 1 up front).
+ *   HVP_CENT_ADOPT (after the solve; reads u [S][n][N], modes [S][n][N], obj, status, nodes [S]): the rollout inputs
+ *       u0 [S][n] = u[s][i][0] and, when gear0 is not NULL, gear0 [S][n] int32 = mode_gear[modes[s][i][0]] (mode
+ *       index clamped to [0, n_modes)).  A scenario whose status is not 2 gets u0 = 0 and gear 6, as
+ *       solve_mpc(raises=False) gives it.  For 0 <= t < T, row t of the episode logs: U_log [T][S][w] = u0, followed
+ *       by the gears as doubles when gear0 is given (w = 2n: the reference's action [u_g ; gears]; else w = n);
+ *       obj_log / status_log / nodes_log [T][S]; aborted_at [S] = the first t whose status is not 2 (-1: none; the
+ *       row is reset at t == 0). */
+#define HVP_CENT_PACK 0
+#define HVP_CENT_ADOPT 1
+typedef struct {
+    int32_t n, N, S, phase;       /* phase: HVP_CENT_PACK | HVP_CENT_ADOPT */
+    int32_t n_param;              /* PACK: length of a params row (hvp_mpc_info[2]), >= 2(N+1) */
+    int32_t leader_per_scenario;  /* PACK: leader_x is [S][2][leader_len] (1) or [2][leader_len] shared (0) */
+    int64_t leader_len;           /* PACK: columns of the leader trajectory (>= 1) */
+    int64_t T;                    /* ADOPT: rows of the episode logs */
+    int32_t n_modes;              /* ADOPT with gear0: entries of mode_gear (1..16) */
+    int32_t reserved;
+    int32_t mode_gear[16];        /* ADOPT with gear0: gear of each mode (hvp_mpc_mode_table) */
+    const int64_t* t;             /* device pointer: timestep index */
+    const double* leader_x;       /* PACK */
+    double* params;               /* PACK: [S][n_param] */
+    const double* u; const int32_t* modes; const double* obj; const int32_t* status; const int32_t* nodes; /* ADOPT in */
+    double* u0; int32_t* gear0;   /* ADOPT out: [S][n] each; gear0 may be NULL */
+    double* U_log; double* obj_log; int32_t* status_log; int32_t* nodes_log; int32_t* aborted_at;   /* ADOPT out */
+} hvp_cent_step;
+int hvp_cent_step_dev(hvp_ctx* ctx, const hvp_cent_step* g, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
