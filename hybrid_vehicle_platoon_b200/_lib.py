@@ -71,7 +71,23 @@ class CentStep(C.Structure):       # hvp_cent_step
                                           "U_log", "obj_log", "status_log", "nodes_log", "aborted_at")]
 
 
+class EventGroup(C.Structure):     # hvp_event_group: the buffers of one group's eval and solve launches
+    _fields_ = [(k, C.c_void_p) for k in ("x0", "xg", "ug", "params", "cost", "u", "x", "modes", "obj", "status", "nodes")] + \
+               [("n_local", C.c_int32), ("n_param", C.c_int32), ("has_leader", C.c_int32), ("reserved", C.c_int32)]
+
+
+class EventIter(C.Structure):      # hvp_event_iter
+    _fields_ = [("n", C.c_int32), ("N", C.c_int32), ("S", C.c_int32), ("phase", C.c_int32), ("iters", C.c_int32),
+                ("it", C.c_int32), ("ngroups", C.c_int32), ("leader_per_scenario", C.c_int32), ("leader_len", C.c_int64),
+                ("T", C.c_int64), ("threshold", C.c_double), ("n_modes", C.c_int32), ("reserved", C.c_int32),
+                ("mode_gear", C.c_int32 * 16), ("group_of", C.c_int32 * 64), ("slot_of", C.c_int32 * 64),
+                ("group", EventGroup * 8)] + \
+               [(k, C.c_void_p) for k in ("t", "x", "leader_x", "SG", "UG", "GG", "active", "WIN", "FEAS", "ND", "U_log",
+                                          "u0", "gear0")]
+
+
 CENT_PACK, CENT_ADOPT = 0, 1
+EVENT_PACK, EVENT_SELECT, EVENT_ADOPT = 0, 1, 2
 MPC_CENT, MPC_LOCAL, MPC_EVENT, MPC_ADMM, MPC_GADMM = 1, 2, 3, 4, 5
 MODEL_PWA_GEAR, MODEL_FRICTION_GEAR = 0, 1
 REAL_VEHICLE_REF, NO_LEADER = 8, -100
@@ -133,6 +149,7 @@ def lib():
     L.hvp_decent_observe_dev.argtypes = [_vp, C.POINTER(DecentObserve), _vp]
     L.hvp_admm_round_dev.argtypes = [_vp, C.POINTER(AdmmRound), _vp]
     L.hvp_cent_step_dev.argtypes = [_vp, C.POINTER(CentStep), _vp]
+    L.hvp_event_iter_dev.argtypes = [_vp, C.POINTER(EventIter), _vp]
     L.hvp_microbench_fp64.argtypes = [_vp, C.c_int, C.POINTER(C.c_double)]
     L.hvp_microbench_smem.argtypes = [_vp, C.c_int, C.POINTER(C.c_double)]
     _lib = L

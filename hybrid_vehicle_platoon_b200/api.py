@@ -238,3 +238,12 @@ def cent_step_device(g, *, phase: int, ctx=None, stream=None):
     ctx = ctx or default_context()
     g.phase = int(phase)
     check(lib().hvp_cent_step_dev(ctx.handle, C.byref(g), _stream_arg(stream)))
+
+
+def event_iter_device(g, *, phase: int, ctx=None, stream=None):
+    """Fused glue of an event-based iteration (hvp_event_iter_dev): phase _lib.EVENT_PACK fills the groups' eval / solve
+    inputs from the guesses, _lib.EVENT_SELECT picks each scenario's winner and adopts its plan, _lib.EVENT_ADOPT takes
+    the first inputs, logs them and shifts the guesses; `g` is a _lib.EventIter."""
+    ctx = ctx or default_context()
+    g.phase = int(phase)
+    check(lib().hvp_event_iter_dev(ctx.handle, C.byref(g), _stream_arg(stream)))

@@ -350,6 +350,146 @@ cent_step_kernel(const __grid_constant__ CentArgs A) {
     }
 }
 
+// ---- event-based controller: the glue of one iteration of TrackingEventBasedCoordinator.get_control and the end of a
+// timestep (fleet_event_based.py:42-107) -------------------------------------------------------------------------------
+struct EvArgs {
+    hvp_event_iter g;
+    int count[8];                     // agents of each group: a group's rows are [scenario][slot]
+    long long lx_sstride;             // leader trajectory scenario stride, 0 when shared
+};
+// agent i optimises the members first..first + nl - 1 ([i-1, i, i+1] clipped at the ends; [0, 1] for both when n = 2)
+__host__ __device__ __forceinline__ int ev_first(int n, int i) { return (n == 2 || i == 0) ? 0 : (i == n - 1 ? n - 2 : i - 1); }
+__host__ __device__ __forceinline__ int ev_nmem(int n, int i) { return (n == 2 || i == 0 || i == n - 1) ? 2 : 3; }
+__device__ __forceinline__ int64_t ev_row(const EvArgs& A, int s, int i) {
+    return (int64_t)s * A.count[A.g.group_of[i]] + A.g.slot_of[i];
+}
+
+__global__ void __launch_bounds__(128)
+event_pack_kernel(const __grid_constant__ EvArgs A) {
+    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = A.g.n, N = A.g.N, np1 = N + 1, blk = 2 * np1;
+    if (tid >= (int64_t)A.g.S * n) return;
+    const int s = (int)(tid / n), i = (int)(tid - (int64_t)s * n);
+    const hvp_event_group& G = A.g.group[A.g.group_of[i]];
+    const int64_t b = ev_row(A, s, i);
+    const int nl = G.n_local, f = ev_first(n, i);
+    for (int l = 0; l < nl; ++l) {
+        const size_t src = (size_t)s * n + f + l, dst = (size_t)b * nl + l;
+        G.x0[2 * dst] = A.g.x[2 * src]; G.x0[2 * dst + 1] = A.g.x[2 * src + 1];
+        for (int e = 0; e < blk; ++e) G.xg[dst * blk + e] = A.g.SG[src * blk + e];
+        for (int k = 0; k < N; ++k) G.ug[dst * N + k] = A.g.UG[src * N + k];
+    }
+    double* P = G.params + (size_t)b * G.n_param;
+    if (G.has_leader) {
+        const long long t = *A.g.t, L = A.g.leader_len;
+        const double* l = A.g.leader_x + (size_t)s * A.lx_sstride;
+        for (int e = 0; e < blk; ++e) {
+            const int row = e / np1;
+            long long c = t + (e - row * np1);
+            c = c < 0 ? 0 : (c >= L ? L - 1 : c);
+            P[e] = l[row * L + c];
+        }
+    } else {
+        for (int e = 0; e < blk; ++e) P[e] = 0.0;
+    }
+    const double* f2 = i > 1 ? A.g.SG + ((size_t)s * n + i - 2) * blk : nullptr;
+    const double* b2 = i < n - 2 ? A.g.SG + ((size_t)s * n + i + 2) * blk : nullptr;
+    for (int e = 0; e < blk; ++e) {
+        P[blk + e] = f2 ? f2[e] : 0.0;
+        P[2 * blk + e] = b2 ? b2[e] : 0.0;
+    }
+}
+
+// one warp per scenario
+__global__ void __launch_bounds__(128)
+event_select_kernel(const __grid_constant__ EvArgs A) {
+    const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    const int n = A.g.n, N = A.g.N, blk = 2 * (N + 1);
+    if (w >= A.g.S) return;
+    const int s = (int)w;
+    if (!A.g.active[s]) return;
+    constexpr int NONE = 1 << 30;
+    constexpr unsigned FULL = 0xffffffffu;
+    double best = -INFINITY;
+    int bi = NONE, nd = INT32_MIN;
+    bool feas = false;
+    for (int i = lane; i < n; i += 32) {
+        const hvp_event_group& G = A.g.group[A.g.group_of[i]];
+        const int64_t b = ev_row(A, s, i);
+        const double c1 = G.status[b] == HVP_OPTIMAL ? G.obj[b] : INFINITY;
+        const double dec = __dadd_rn(G.cost[b], -c1);       // inf - inf = NaN: never > threshold
+        feas |= (bool)isfinite(c1);
+        nd = max(nd, G.nodes[b]);
+        if (dec > A.g.threshold && (bi == NONE || dec > best)) { best = dec; bi = i; }
+    }
+    // largest decrease, the first agent among equal ones
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ob = __shfl_xor_sync(FULL, best, o);
+        const int oi = __shfl_xor_sync(FULL, bi, o);
+        if (oi != NONE && (bi == NONE || ob > best || (ob == best && oi < bi))) { best = ob; bi = oi; }
+        nd = max(nd, __shfl_xor_sync(FULL, nd, o));
+    }
+    feas = __any_sync(FULL, feas);
+    const long long t = *A.g.t;
+    if (lane == 0 && t >= 0 && t < A.g.T) {
+        const size_t r = (size_t)t * A.g.S + s;
+        if (!feas) A.g.FEAS[r] = 0;
+        A.g.ND[r] = max(A.g.ND[r], nd);
+        A.g.WIN[r * A.g.iters + A.g.it] = bi == NONE ? -1 : bi;
+    }
+    if (bi == NONE) {                 // nobody improved: the reference stops iterating this timestep
+        if (lane == 0) A.g.active[s] = 0;
+        return;
+    }
+    // the winner's plan overwrites the shared guesses of its members
+    const hvp_event_group& G = A.g.group[A.g.group_of[bi]];
+    const int64_t b = ev_row(A, s, bi);
+    const int nl = G.n_local;
+    const size_t base = (size_t)s * n + ev_first(n, bi);
+    for (int e = lane; e < nl * blk; e += 32) {
+        const int l = e / blk;
+        A.g.SG[(base + l) * blk + (e - l * blk)] = G.x[(size_t)b * nl * blk + e];
+    }
+    for (int e = lane; e < nl * N; e += 32) {
+        const int l = e / N;
+        const size_t d = (base + l) * N + (e - l * N);
+        A.g.UG[d] = G.u[(size_t)b * nl * N + e];
+        if (A.g.GG) {
+            int m = G.modes[(size_t)b * nl * N + e];
+            m = m < 0 ? 0 : (m >= A.g.n_modes ? A.g.n_modes - 1 : m);
+            A.g.GG[d] = A.g.mode_gear[m];
+        }
+    }
+}
+
+__global__ void __launch_bounds__(128)
+event_adopt_kernel(const __grid_constant__ EvArgs A) {
+    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int n = A.g.n, N = A.g.N, np1 = N + 1;
+    if (tid >= (int64_t)A.g.S * n) return;
+    const int s = (int)(tid / n), i = (int)(tid - (int64_t)s * n);
+    double* sg = A.g.SG + (size_t)tid * 2 * np1;
+    double* ug = A.g.UG + (size_t)tid * N;
+    int32_t* gg = A.g.GG ? A.g.GG + (size_t)tid * N : nullptr;
+    const double u0 = ug[0];
+    A.g.u0[tid] = u0;
+    if (gg) A.g.gear0[tid] = gg[0];
+    const long long t = *A.g.t;
+    if (t >= 0 && t < A.g.T) {
+        double* Ur = A.g.U_log + ((size_t)t * A.g.S + s) * (gg ? 2 * n : n);
+        Ur[i] = u0;
+        if (gg) Ur[n + i] = (double)gg[0];
+    }
+    // shifted previous solution: drop column 0, repeat the last one (fleet_event_based.py:98-103)
+    for (int k = 0; k < N; ++k) { sg[k] = sg[k + 1]; sg[np1 + k] = sg[np1 + k + 1]; }
+    for (int k = 0; k + 1 < N; ++k) {
+        ug[k] = ug[k + 1];
+        if (gg) gg[k] = gg[k + 1];
+    }
+    if (i == 0) A.g.active[s] = 1;
+}
+
 }  // namespace hvp
 
 using namespace hvp;
@@ -489,6 +629,72 @@ extern "C" int hvp_cent_step_dev(hvp_ctx* c, const hvp_cent_step* g, void* strea
     cent_step_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(A);
     e = cudaGetLastError();
     if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "cent_step: launch failed: %s", cudaGetErrorString(e));
+    c->launches += 1;
+    return 0;
+}
+
+// hvp.h: hvp_event_iter_dev
+extern "C" int hvp_event_iter_dev(hvp_ctx* c, const hvp_event_iter* g, void* stream) {
+    if (!c || !g) return hvp_fail(-1, "event_iter: NULL argument");
+    const int n = g->n, ph = g->phase;
+    if (n < 2 || n > 64 || g->N < 1 || g->S < 0 || (ph != HVP_EVENT_PACK && ph != HVP_EVENT_SELECT && ph != HVP_EVENT_ADOPT))
+        return hvp_fail(-4, "event_iter: bad sizes (n=%d N=%d S=%d phase=%d)", n, g->N, g->S, ph);
+    if (g->ngroups < 1 || g->ngroups > 8 || g->iters < 1 || g->it < 0 || g->it >= g->iters || g->T < 0 ||
+        (g->GG && (g->n_modes < 1 || g->n_modes > 16)))
+        return hvp_fail(-4, "event_iter: bad sizes (groups=%d it=%d iters=%d T=%lld n_modes=%d)", g->ngroups, g->it, g->iters,
+                        (long long)g->T, g->n_modes);
+    EvArgs A;
+    A.g = *g;
+    uint64_t seen[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    for (int r = 0; r < 8; ++r) A.count[r] = 0;
+    for (int i = 0; i < n; ++i) {
+        const int r = g->group_of[i], k = g->slot_of[i];
+        if (r < 0 || r >= g->ngroups || k < 0 || k >= 64 || (seen[r] >> k & 1))
+            return hvp_fail(-4, "event_iter: agent %d has group %d slot %d (out of range or taken)", i, r, k);
+        if (g->group[r].n_local != ev_nmem(n, i))
+            return hvp_fail(-4, "event_iter: group %d has %d members per agent, agent %d has %d", r, g->group[r].n_local, i,
+                            ev_nmem(n, i));
+        seen[r] |= 1ull << k;
+        A.count[r] += 1;
+    }
+    for (int i = 0; i < n; ++i)       // the slots of a group are 0 .. count - 1
+        if (g->slot_of[i] >= A.count[g->group_of[i]])
+            return hvp_fail(-4, "event_iter: agent %d has slot %d of a group of %d", i, g->slot_of[i], A.count[g->group_of[i]]);
+    bool lead = false;
+    for (int r = 0; r < g->ngroups; ++r) {
+        if (A.count[r] == 0) continue;
+        const hvp_event_group& G = g->group[r];
+        lead |= G.has_leader != 0;
+        if (ph == HVP_EVENT_PACK && G.n_param < 6 * (g->N + 1))
+            return hvp_fail(-4, "event_iter: group %d n_param=%d < 6(N+1)", r, G.n_param);
+    }
+    if (ph == HVP_EVENT_PACK && lead && g->leader_len < 1)
+        return hvp_fail(-4, "event_iter: bad sizes (leader_len=%lld)", (long long)g->leader_len);
+    if (g->S == 0) return 0;
+    if (!g->t || !g->SG || !g->UG) return hvp_fail(-1, "event_iter: NULL array argument");
+    for (int r = 0; r < g->ngroups; ++r) {
+        const hvp_event_group& G = g->group[r];
+        if (A.count[r] == 0) continue;
+        if (ph == HVP_EVENT_PACK && (!G.x0 || !G.xg || !G.ug || !G.params))
+            return hvp_fail(-1, "event_iter: NULL group buffer (pack, group %d)", r);
+        if (ph == HVP_EVENT_SELECT && (!G.cost || !G.u || !G.x || !G.obj || !G.status || !G.nodes || (g->GG && !G.modes)))
+            return hvp_fail(-1, "event_iter: NULL group buffer (select, group %d)", r);
+    }
+    if ((ph == HVP_EVENT_PACK && (!g->x || (lead && !g->leader_x))) ||
+        (ph == HVP_EVENT_SELECT && (!g->active || !g->WIN || !g->FEAS || !g->ND)) ||
+        (ph == HVP_EVENT_ADOPT && (!g->active || !g->U_log || !g->u0 || (g->GG && !g->gear0))))
+        return hvp_fail(-1, "event_iter: NULL array argument (phase %d)", ph);
+    A.lx_sstride = g->leader_per_scenario ? 2 * g->leader_len : 0;
+    cudaError_t e = cudaSetDevice(c->device);
+    if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "event_iter: cudaSetDevice: %s", cudaGetErrorString(e));
+    cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
+    const int64_t threads = (int64_t)g->S * (ph == HVP_EVENT_SELECT ? 32 : n);
+    const unsigned blocks = (unsigned)((threads + 127) / 128);
+    if (ph == HVP_EVENT_PACK) event_pack_kernel<<<blocks, 128, 0, st>>>(A);
+    else if (ph == HVP_EVENT_SELECT) event_select_kernel<<<blocks, 128, 0, st>>>(A);
+    else event_adopt_kernel<<<blocks, 128, 0, st>>>(A);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "event_iter: launch failed: %s", cudaGetErrorString(e));
     c->launches += 1;
     return 0;
 }

@@ -6,7 +6,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from ._sim import collect, make_env_and_systems
+from ._sim import collect, make_env_and_systems, save_results
 from .agents import MldAgent
 from .misc import Params, Sim
 from .mpc import EventLocalMpc as LocalMpc, eval_compiled_batch, solve_compiled_batch
@@ -149,3 +149,57 @@ def simulate(sim: Sim, event_iters: int = 4, save: bool = False, plot: bool = Fa
                                           leader_index=leader_index)
     agent.evaluate(env=env, episodes=1, seed=seed)
     return collect(env, agent, leader_x, f"event_{event_iters}_{sim.id}_seed_{seed}.pkl", save)
+
+
+def simulate_many(sim: Sim, seeds, event_iters: int = 4, leader_index: int = 0, ep_len=None, save: bool = False,
+                  strict: bool = True, ctx=None):
+    """simulate() for several seeds of one configuration in ONE on-device closed loop (sweep.BatchedEventSweep): the
+    paper's "10 seeds of a configuration" in one call.  Each seed's initial state is PlatoonEnv.reset with the seed
+    MldAgent.evaluate derives from it, the masses are the env's and the solver options are the ones simulate() would use
+    (mpc.OPTIONS).  Returns one dict per seed with simulate()'s 7 objects and shapes, except solve_times, which is NaN: a
+    batched launch has no per-scenario solve time; node_counts is the largest node count over the iterations and agents
+    of a timestep.  save=True writes simulate()'s pickle per seed.  strict=True raises what simulate() would after the
+    run, naming the seed and timestep: RuntimeWarning for an iteration in which no agent's MIQP was solved, the rollout's
+    error otherwise; strict=False returns the episodes as computed."""
+    from .env import raise_rollout_error
+    from .mpc import OPTIONS
+    from .sweep import BatchedEventSweep
+    n, N = sim.n, sim.N
+    if n < 2:
+        raise ValueError("the event-based scheme needs at least two vehicles")
+    seeds = [int(s) for s in seeds]
+    leader_x = sim.leader_trajectory.get_leader_trajectory()
+    env, _, _, ep_len = make_env_and_systems(sim, leader_index, ep_len, None, forward_real_ref=False)
+    base = env.unwrapped
+    x0 = np.stack([np.asarray(env.reset(seed=int(np.random.SeedSequence(s).generate_state(1)[0]))[0],
+                              dtype=np.float64).reshape(2 * n) for s in seeds])
+    sw = BatchedEventSweep(n, N, event_iters=event_iters, masses=base.masses, spacing_policy=sim.spacing_policy,
+                           leader_index=leader_index, d_safe=base.d_safe, threshold=threshold, model=sim.vehicle_model_type,
+                           mip_gap=OPTIONS.mip_gap, time_limit_ms=OPTIONS.time_limit * 1e3, ctx=ctx)
+    try:
+        r = sw.run(x0, leader_x, ep_len)
+    finally:
+        sw.close()
+    if strict:
+        # what simulate() meets first in each episode; the first episode (in seed order) that meets one is reported
+        for j, seed in enumerate(seeds):
+            bad_t = np.nonzero(~r["feasible"][:, j])[0]
+            err_t = np.nonzero(r["errors"][:, j])[0]
+            if bad_t.size and (not err_t.size or bad_t[0] <= err_t[0]):
+                raise RuntimeWarning(f"No feasible solution found for any event based agent. (seed {seed}, timestep "
+                                     f"{int(bad_t[0])})")
+            if err_t.size:
+                try:
+                    raise_rollout_error(int(r["errors"][err_t[0], j]))
+                except RuntimeError as e:
+                    raise RuntimeError(f"{e} (seed {seed}, timestep {int(err_t[0])})") from None
+    out = []
+    for j, seed in enumerate(seeds):
+        # shapes of collect(): X (T+1,2n), U (T,n|2n), R (T,1,1), solve_times / node_counts (T,1), violations (T,)
+        res = dict(X=r["X"][:, j].copy(), U=r["U"][:, j].copy(), R=r["R"][:, j].reshape(ep_len, 1, 1).copy(),
+                   solve_times=np.full((ep_len, 1), np.nan), node_counts=r["nodes"][:, j].astype(np.float64).reshape(ep_len, 1),
+                   violations=np.where(r["violations"][:, j] != 0, 100.0, 0.0), leader_x=leader_x)
+        if save:
+            save_results(res, f"event_{event_iters}_{sim.id}_seed_{seed}.pkl")
+        out.append(res)
+    return out

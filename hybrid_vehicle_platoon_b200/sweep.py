@@ -1088,20 +1088,68 @@ class BatchedGAdmmSweep:
                     aborted_at=aborted_at, best_warm_start=WS.cpu().numpy())
 
 
+def friction_gear_from_velocity(v):
+    """PwaFrictionVehicle.get_gear_from_velocity over a float64 torch tensor of velocities (any device): gear 1 below
+    v_min, 6 above v_max, else the first gear whose OPEN window (vl, vh) contains v.  0 where the scalar method raises
+    (v on an end of the velocity range that no open window contains)."""
+    import torch
+    from .models import Vehicle
+    g = torch.zeros(v.shape, dtype=torch.int64, device=v.device)
+    for i in reversed(range(len(Vehicle.b))):
+        g = torch.where((Vehicle.vl[i] < v) & (v < Vehicle.vh[i]), i + 1, g)
+    g = torch.where(v > Vehicle.v_max, 6, g)
+    return torch.where(v < Vehicle.v_min, 1, g)
+
+
+def friction_const_vel_u(v, gear, mass):
+    """PwaFrictionVehicle.get_u_for_constant_vel(v, gear) over torch tensors of the same shape (any device), in the
+    scalar method's order of operations: (1 / (b_j * (1 / m))) * (-A_r[1, 1] v - c_r[1]) with friction region
+    r = 0 for v <= alpha, else 1."""
+    import torch
+    from .models import PwaFrictionVehicle as V
+    f64 = torch.float64
+    b = torch.tensor(V.b, dtype=f64, device=v.device)[gear - 1]
+    hi = v > V.alpha
+    # tensor / tensor only: torch evaluates `scalar / tensor` as a reciprocal times the scalar (two roundings)
+    a = -(-torch.tensor([V.c1, V.c2], dtype=f64, device=v.device)[hi.long()] / mass)
+    mug = -V.mu * V.grav
+    c = torch.where(hi, mug - torch.full_like(mass, V.d) / mass, torch.full_like(mass, mug))
+    return (1 / (b * (1 / mass))) * (a * v - c)
+
+
 class BatchedEventSweep:
     """S independent platoons under the event-based controller (fleet_event_based.py:413-646), state and guesses
     resident on the device.  One iteration = for every distinct local formulation (agents grouped by vehicles in
     front / behind and relative leader position) ONE eval_cost launch and ONE MIQP launch over S x agents problems,
     then the winner selection (largest cost decrease above `threshold`, first agent on ties) and the overwrite of
-    the shared guesses as torch ops.  Scenarios whose iteration found no improver are left unchanged by the
-    remaining iterations (the same solves repeat), which is the reference's `break`."""
+    the shared guesses.  A scenario whose iteration found no improver is left unchanged by the remaining iterations of
+    the timestep, which is the reference's `break`.
+
+    model: "pwa_gear" (gears derived from the velocities) or "pwa_friction" (discrete gears chosen by the MPC; the
+    action is [u_g ; gears]).  fused: the glue of an iteration as the three phases of ONE kernel (hvp_event_iter_dev,
+    csrc/coord.cu), with no host synchronisation until the results are read back; None reads HVP_SWEEP_FUSED (default
+    on).  fused=False keeps the glue as torch ops, pwa_gear only: the reference the kernel is tested against.
+    fork / graph (fused loop): the groups' eval and solve launches on forked streams / each iteration replayed as a CUDA
+    graph; off by default, the A/B arms of scripts/time_event_sweep.py (DESIGN.md 5b)."""
 
     def __init__(self, n: int, N: int, event_iters: int = 4, masses=None, spacing_policy=ConstantSpacingPolicy(50),
-                 leader_index: int = 0, d_safe: float = Params.d_safe, threshold: float = 10.0, device: int = 0, ctx=None):
+                 leader_index: int = 0, d_safe: float = Params.d_safe, threshold: float = 10.0, model: str = "pwa_gear",
+                 mip_gap: float = 0.0, time_limit_ms: float = 0.0, device: int = 0, ctx=None, fused=None,
+                 fork: bool = False, graph: bool = False):
+        import os
         import torch
-        from ._lib import MPC_EVENT, NO_LEADER
+        from ._lib import MODEL_FRICTION_GEAR, MODEL_PWA_GEAR, MPC_EVENT, NO_LEADER
+        self.fork, self.graph = fork, graph
+        if model not in ("pwa_gear", "pwa_friction"):
+            raise ValueError(f"model must be 'pwa_gear' or 'pwa_friction', got {model!r}")
+        self.fused = (os.environ.get("HVP_SWEEP_FUSED", "1") != "0") if fused is None else bool(fused)
+        self.friction = model == "pwa_friction"
+        if self.friction and not self.fused:
+            raise ValueError("the torch glue (fused=False) runs the pwa_gear model only")
         if n < 2:
             raise ValueError("the event-based scheme needs at least two vehicles")
+        if self.fused and (n > 64 or event_iters < 1):
+            raise ValueError(f"the fused loop needs n <= 64 and event_iters >= 1 (n = {n}, event_iters = {event_iters})")
         self.torch, self.n, self.N, self.iters, self.leader_index = torch, n, N, event_iters, leader_index
         self.threshold = float(threshold)
         self.dev = torch.device("cuda", device)
@@ -1121,8 +1169,9 @@ class BatchedEventSweep:
             groups.setdefault((nf, nb, rl, len(self.members[i])), []).append(i)
         self.groups = []
         for (nf, nb, rl, nl), idx in groups.items():
-            cm = api.CompiledMpc(MPC_EVENT, N, n_local=nl, leader_index=NO_LEADER if rl is None else rl, n_front=nf,
-                                 n_behind=nb, d0=self.d0, t0=self.t0, ctx=self.ctx)
+            cm = api.CompiledMpc(MPC_EVENT, N, n_local=nl, model=MODEL_FRICTION_GEAR if self.friction else MODEL_PWA_GEAR,
+                                 leader_index=NO_LEADER if rl is None else rl, n_front=nf, n_behind=nb, d0=self.d0,
+                                 t0=self.t0, mip_gap=mip_gap, time_limit_ms=time_limit_ms, ctx=self.ctx)
             self.groups.append((cm, idx, nl, nf, nb, rl))
         from .models import PwaGearVehicle
         v = PwaGearVehicle(800.0)
@@ -1137,23 +1186,50 @@ class BatchedEventSweep:
 
     _const_vel_u = BatchedGAdmmSweep._const_vel_u
 
+    def close(self):
+        """Releases the compiled formulations (their device scratch)."""
+        for cm, *_ in self.groups:
+            cm.close()
+        self.groups = []
+
     def run(self, x0, leader_x, ep_len: int):
-        """Returns dict of numpy arrays: X (T+1,S,2n), U (T,S,n), R (T,S), violations, errors, winners
-        (T,S,event_iters) int32 (-1: nobody improved), feasible (T,S) bool, nodes (T,S) int32 (max over agents)."""
+        """x0 (S,2n) initial states, leader_x (2,>=ep_len+N+1) shared or (S,2,>=ep_len+N+1) per scenario.  Returns dict
+        of numpy arrays: X (T+1,S,2n), U (T,S,n) -- (T,S,2n) = [u_g ; gears] for pwa_friction --, R (T,S), violations,
+        errors, winners (T,S,event_iters) int32 (-1: nobody improved, or the scenario had stopped iterating), feasible
+        (T,S) bool (False: an iteration in which no agent's MIQP was solved, where simulate() raises), nodes (T,S) int32
+        (max over iterations and agents)."""
         torch, dev, n, N = self.torch, self.dev, self.n, self.N
         f64, i32, np1 = torch.float64, torch.int32, N + 1
-        x = torch.as_tensor(np.ascontiguousarray(x0, dtype=np.float64), device=dev)
-        S = x.shape[0]
-        lx = torch.as_tensor(np.ascontiguousarray(leader_x, dtype=np.float64), device=dev)
-        if lx.ndim == 2:
-            lx = lx.unsqueeze(0).expand(S, -1, -1)
-        if lx.shape[2] < ep_len + np1:
+        if not self.groups:
+            raise RuntimeError("BatchedEventSweep is closed")
+        x0 = np.ascontiguousarray(x0, dtype=np.float64)
+        if x0.ndim != 2 or x0.shape[1] != 2 * n:
+            raise ValueError(f"x0 must have shape (S, {2 * n}), got {x0.shape}")
+        S = x0.shape[0]
+        lx_np = np.ascontiguousarray(leader_x, dtype=np.float64)
+        if lx_np.ndim not in (2, 3) or lx_np.shape[-2] != 2 or (lx_np.ndim == 3 and lx_np.shape[0] != S):
+            raise ValueError(f"leader_x must have shape (2, L) or ({S}, 2, L), got {lx_np.shape}")
+        if lx_np.shape[-1] < ep_len + np1:
             raise ValueError("leader trajectory shorter than ep_len + N + 1")
         m = np.full((S, n), 800.0) if self.masses is None else np.broadcast_to(self.masses, (S, n))
-        mass = torch.as_tensor(np.array(m, dtype=np.float64, order="C"), device=dev)
+        m = np.array(m, dtype=np.float64, order="C")
+        # first guesses: constant velocity, constant-velocity throttle (fleet_event_based.py:620-634); with discrete
+        # gears the gear of the velocity and the throttle in that gear, computed on the host before anything is queued
+        gear = None
+        if self.friction:
+            v_h, m_h = torch.as_tensor(x0[:, 1::2]), torch.as_tensor(m)
+            gear = friction_gear_from_velocity(v_h)
+            if (gear == 0).any():
+                s_, i_ = (int(a) for a in torch.nonzero(gear == 0)[0])
+                raise ValueError(f"No gear found for velocity {x0[s_, 2 * i_ + 1]} (scenario {s_}, vehicle {i_})")
+            u_first = friction_const_vel_u(v_h, gear, m_h)
+        x = torch.as_tensor(x0, device=dev)
+        lx = torch.as_tensor(lx_np, device=dev)
+        mass = torch.as_tensor(m, device=dev)
         edesc = api.env_desc(n, self.leader_index, self.d0, self.t0, self.d_safe, True, False, True)
+        w = 2 * n if self.friction else n
         X = torch.empty((ep_len + 1, S, 2 * n), dtype=f64, device=dev)
-        U = torch.empty((ep_len, S, n), dtype=f64, device=dev)
+        U = torch.empty((ep_len, S, w), dtype=f64, device=dev)
         R = torch.empty((ep_len, S), dtype=f64, device=dev)
         V = torch.empty((ep_len, S), dtype=torch.uint8, device=dev)
         E = torch.empty((ep_len, S), dtype=i32, device=dev)
@@ -1161,16 +1237,115 @@ class BatchedEventSweep:
         FEAS = torch.ones((ep_len, S), dtype=torch.bool, device=dev)
         ND = torch.zeros((ep_len, S), dtype=i32, device=dev)
         X[0] = x
-        stream = torch.cuda.current_stream().cuda_stream
         ts = float(Params.ts)
-        # first guesses: constant velocity, constant-velocity throttle (fleet_event_based.py:620-634)
         xv = x.view(S, n, 2)
         SG = torch.empty((S, n, 2, np1), dtype=f64, device=dev)
         SG[:, :, 0, 0] = xv[:, :, 0]
         SG[:, :, 1, :] = xv[:, :, 1:2]
         for k in range(N):
             SG[:, :, 0, k + 1] = SG[:, :, 0, k] + ts * SG[:, :, 1, k]
-        UG = self._const_vel_u(x, mass).unsqueeze(-1).expand(S, n, N).contiguous()
+        if self.friction:
+            UG = u_first.to(dev).unsqueeze(-1).expand(S, n, N).contiguous()
+            GG = gear.to(device=dev, dtype=i32).unsqueeze(-1).expand(S, n, N).contiguous()
+        else:
+            UG = self._const_vel_u(x, mass).unsqueeze(-1).expand(S, n, N).contiguous()
+            GG = None
+        logs = (X, U, R, V, E, WIN, FEAS, ND)
+        if self.fused:
+            self._run_fused(S, ep_len, x, lx, mass, edesc, SG, UG, GG, logs)
+        else:
+            self._run_torch(S, ep_len, x, lx, mass, edesc, SG, UG, logs)
+        torch.cuda.synchronize()
+        return dict(X=X.cpu().numpy(), U=U.cpu().numpy(), R=R.cpu().numpy(), violations=V.cpu().numpy(),
+                    errors=E.cpu().numpy(), winners=WIN.cpu().numpy(), feasible=FEAS.cpu().numpy(), nodes=ND.cpu().numpy())
+
+    def _run_fused(self, S, ep_len, x, lx, mass, edesc, SG, UG, GG, logs):
+        from . import _lib
+        torch, dev, n, N = self.torch, self.dev, self.n, self.N
+        f64, i32, np1 = torch.float64, torch.int32, N + 1
+        X, U, R, V, E, WIN, FEAS, ND = logs
+        g = _lib.EventIter()
+        g.n, g.N, g.S, g.iters, g.ngroups = n, N, S, self.iters, len(self.groups)
+        g.leader_per_scenario, g.leader_len, g.T, g.threshold = int(lx.ndim == 3), lx.shape[-1], ep_len, self.threshold
+        table = self.groups[0][0].mode_gear
+        g.n_modes = len(table)
+        for k, gear in enumerate(table.tolist()):
+            g.mode_gear[k] = gear
+        # eval / solve buffers of every group, allocated once per run; rows [scenario][agent of the group]
+        bufs = []
+        for gi, (cm, idx, nl, nf, nb, rl) in enumerate(self.groups):
+            B = S * len(idx)
+            mm = torch.as_tensor([self.members[i] for i in idx], device=dev)
+            e = lambda *s, dt=f64: torch.empty(s, dtype=dt, device=dev)
+            b = dict(cm=cm, B=B, x0=e(B, nl, 2), xg=e(B, nl, 2, np1), ug=e(B, nl, N),
+                     params=torch.zeros((B, cm.n_param), dtype=f64, device=dev),
+                     m=mass[:, mm].reshape(B, nl).contiguous(), cost=e(B), u=e(B, nl, N), x=e(B, nl, 2, np1),
+                     modes=e(B, nl, N, dt=i32), obj=e(B), status=e(B, dt=i32), nodes=e(B, dt=i32))
+            bufs.append(b)
+            G = g.group[gi]
+            for k in ("x0", "xg", "ug", "params", "cost", "u", "x", "modes", "obj", "status", "nodes"):
+                setattr(G, k, b[k].data_ptr())
+            G.n_local, G.n_param, G.has_leader = nl, cm.n_param, int(rl is not None)
+            for slot, i in enumerate(idx):
+                g.group_of[i], g.slot_of[i] = gi, slot
+        t_idx = torch.zeros(1, dtype=torch.int64, device=dev)
+        active = torch.ones(S, dtype=torch.uint8, device=dev)
+        u0 = torch.empty((S, n), dtype=f64, device=dev)
+        gear0 = torch.empty((S, n), dtype=i32, device=dev) if GG is not None else None
+        lead_t = torch.empty((S, 2), dtype=f64, device=dev)
+        x_cur = x.clone(); x_next = torch.empty_like(x_cur)
+        r_t = torch.empty(S, dtype=f64, device=dev); v_t = torch.empty(S, dtype=torch.uint8, device=dev)
+        e_t = torch.empty(S, dtype=i32, device=dev)
+        ptr = lambda t_: None if t_ is None else t_.data_ptr()
+        g.t, g.x, g.leader_x, g.SG, g.UG, g.GG = t_idx.data_ptr(), x_cur.data_ptr(), lx.data_ptr(), SG.data_ptr(), \
+            UG.data_ptr(), ptr(GG)
+        g.active, g.WIN, g.FEAS, g.ND, g.U_log = active.data_ptr(), WIN.data_ptr(), FEAS.data_ptr(), ND.data_ptr(), U.data_ptr()
+        g.u0, g.gear0 = u0.data_ptr(), ptr(gear0)
+
+        def piece(b):
+            def run_group():
+                stream = torch.cuda.current_stream().cuda_stream
+                b["cm"].eval_device(b["B"], b["m"], b["params"], b["xg"], b["ug"], b["cost"], stream=stream)
+                b["cm"].solve_device(b["B"], b["x0"], b["m"], b["params"], None, b["u"], b["x"], None, b["modes"], b["obj"],
+                                     b["status"], b["nodes"], None, stream=stream)
+            return run_group
+        fork = _Fork(torch, len(bufs), enabled=self.fork)
+        pieces = [piece(b) for b in bufs]
+
+        def iteration(it):
+            def body():
+                stream = torch.cuda.current_stream().cuda_stream
+                g.it = it
+                api.event_iter_device(g, phase=_lib.EVENT_PACK, ctx=self.ctx, stream=stream)
+                fork.run(pieces)
+                api.event_iter_device(g, phase=_lib.EVENT_SELECT, ctx=self.ctx, stream=stream)
+            return _StepGraph(torch, body, enabled=self.graph)
+        iterations = [iteration(it) for it in range(self.iters)]
+
+        stream = torch.cuda.current_stream().cuda_stream
+        for _ in range(ep_len):
+            for step in iterations:
+                step()
+            api.event_iter_device(g, phase=_lib.EVENT_ADOPT, ctx=self.ctx, stream=stream)
+            lead_t.copy_(lx.index_select(-1, t_idx).squeeze(-1))                             # leader_x[:, t]
+            api.rollout_step_device(edesc, S, x_cur, u0, gear0, mass, lead_t, x_next, r_t, v_t, e_t, ctx=self.ctx,
+                                    stream=stream)
+            X.index_copy_(0, t_idx + 1, x_next.unsqueeze(0))
+            R.index_copy_(0, t_idx, r_t.unsqueeze(0))
+            V.index_copy_(0, t_idx, v_t.unsqueeze(0)); E.index_copy_(0, t_idx, e_t.unsqueeze(0))
+            x_cur.copy_(x_next)
+            t_idx.add_(1)
+        torch.cuda.synchronize()
+        for step in iterations:
+            step.close()
+
+    def _run_torch(self, S, ep_len, x, lx, mass, edesc, SG, UG, logs):
+        torch, dev, n, N = self.torch, self.dev, self.n, self.N
+        f64, i32, np1 = torch.float64, torch.int32, N + 1
+        X, U, R, V, E, WIN, FEAS, ND = logs
+        if lx.ndim == 2:
+            lx = lx.unsqueeze(0).expand(S, -1, -1)
+        stream = torch.cuda.current_stream().cuda_stream
         mem = torch.full((n, 3), -1, dtype=torch.int64, device=dev)
         for i, ms in enumerate(self.members):
             mem[i, :len(ms)] = torch.as_tensor(ms, device=dev)
@@ -1227,9 +1402,6 @@ class BatchedEventSweep:
             x = X[t + 1]
             SG = torch.cat((SG[..., 1:], SG[..., -1:]), dim=-1)        # shifted previous solution (:591-603)
             UG = torch.cat((UG[..., 1:], UG[..., -1:]), dim=-1)
-        torch.cuda.synchronize()
-        return dict(X=X.cpu().numpy(), U=U.cpu().numpy(), R=R.cpu().numpy(), violations=V.cpu().numpy(),
-                    errors=E.cpu().numpy(), winners=WIN.cpu().numpy(), feasible=FEAS.cpu().numpy(), nodes=ND.cpu().numpy())
 
 
 class BatchedCentSweep:

@@ -345,6 +345,62 @@ typedef struct {
 } hvp_cent_step;
 int hvp_cent_step_dev(hvp_ctx* ctx, const hvp_cent_step* g, void* stream);
 
+/* ---- fused glue of an event-based iteration ------------------------------------------------------------------
+ * What TrackingEventBasedCoordinator.get_control / on_timestep_end (fleet_event_based.py:42-107) do around the eval
+ * and solve launches, for all S scenarios at once.  Agent i optimises its members m = [i-1, i, i+1] clipped at the
+ * ends ([0, 1] for both agents when n = 2); agents with the same formulation form a group (one eval and one solve
+ * launch each), whose rows are ordered [scenario][agent of the group]: agent i is row s * count + slot_of[i] of
+ * group[group_of[i]], count = the number of agents with that group.  t is read from DEVICE memory.  Three phases:
+ *   HVP_EVENT_PACK   (before the group launches; one thread per (scenario, agent)): x0[row][l] = x[s][m_l],
+ *       xg[row][l] = SG[s][m_l], ug[row][l] = UG[s][m_l], and the parameter blocks [leader_x[:, t : t+N+1] if the
+ *       group has a leader else 0 | SG[s][i-2] if i > 1 else 0 | SG[s][i+2] if i < n-2 else 0] (columns past the end
+ *       of leader_x read its last column).  The rest of a params row is left alone.
+ *   HVP_EVENT_SELECT (after the group launches; one warp per scenario; nothing for a scenario with active[s] == 0):
+ *       cost0 = eval cost, cost1 = obj if status == 2 else +inf, dec = cost0 - cost1 (IEEE: inf - inf is NaN, never
+ *       valid); the winner is the FIRST agent with the largest dec among those with dec > threshold.
+ *       FEAS[t][s] &= any(isfinite(cost1)), ND[t][s] = max(ND[t][s], nodes of every agent), WIN[t][s][it] = winner or
+ *       -1.  The winner's x / u (and, with GG, mode_gear[modes], mode index clamped to [0, n_modes)) overwrite
+ *       SG / UG / GG of its members; no winner sets active[s] = 0 (the reference's `break`).
+ *   HVP_EVENT_ADOPT  (after the last iteration, before the rollout; one thread per (scenario, agent)): u0 = UG[:, :, 0],
+ *       gear0 = GG[:, :, 0] with gears, U_log[t] = u0 (then the gears as doubles: w = 2n), SG / UG / GG shifted one
+ *       column left repeating the last one, active[s] = 1.
+ * Log rows are written only for 0 <= t < T.  All pointers are device pointers. */
+#define HVP_EVENT_PACK 0
+#define HVP_EVENT_SELECT 1
+#define HVP_EVENT_ADOPT 2
+typedef struct {
+    double* x0; double* xg; double* ug; double* params;  /* PACK out: [rows][nl][2], [rows][nl][2][N+1], [rows][nl][N], [rows][n_param] */
+    const double* cost; /* SELECT in: eval output [rows] */
+    const double* u; const double* x; const int32_t* modes; const double* obj; const int32_t* status; const int32_t* nodes; /* SELECT in: solve output */
+    int32_t n_local;    /* members of each agent of the group (2 or 3) */
+    int32_t n_param;    /* >= 6(N+1) */
+    int32_t has_leader; /* the group's formulation has a relative leader (parameter block 0) */
+    int32_t reserved;
+} hvp_event_group;
+typedef struct {
+    int32_t n, N, S, phase;       /* phase: HVP_EVENT_PACK | HVP_EVENT_SELECT | HVP_EVENT_ADOPT */
+    int32_t iters, it;            /* SELECT: iterations per timestep, this iteration (the WIN column) */
+    int32_t ngroups;              /* 1..8 */
+    int32_t leader_per_scenario;  /* PACK: leader_x is [S][2][leader_len] (1) or [2][leader_len] shared (0) */
+    int64_t leader_len;           /* PACK: columns of the leader trajectory (>= 1) */
+    int64_t T;                    /* SELECT / ADOPT: rows of the episode logs */
+    double threshold;             /* SELECT: least cost decrease of a winner (exclusive) */
+    int32_t n_modes;              /* SELECT with GG: entries of mode_gear (1..16) */
+    int32_t reserved;
+    int32_t mode_gear[16];
+    int32_t group_of[64], slot_of[64];
+    hvp_event_group group[8];
+    const int64_t* t;             /* device pointer: timestep index */
+    const double* x;              /* PACK: [S][n][2] */
+    const double* leader_x;       /* PACK */
+    double* SG; double* UG; int32_t* GG;   /* guesses [S][n][2][N+1], [S][n][N], [S][n][N] (GG NULL: pwa_gear) */
+    uint8_t* active;              /* [S] */
+    int32_t* WIN; uint8_t* FEAS; int32_t* ND;  /* SELECT logs [T][S][iters], [T][S], [T][S] */
+    double* U_log;                /* ADOPT log [T][S][w] */
+    double* u0; int32_t* gear0;   /* ADOPT out [S][n] each; gear0 with GG only */
+} hvp_event_iter;
+int hvp_event_iter_dev(hvp_ctx* ctx, const hvp_event_iter* g, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
