@@ -86,8 +86,23 @@ class EventIter(C.Structure):      # hvp_event_iter
                                           "u0", "gear0")]
 
 
+class AdmmStepRole(C.Structure):   # hvp_admm_step_role: the buffers of one role's solve launch
+    _fields_ = [(k, C.c_void_p) for k in ("params", "x0", "u", "x", "extra", "modes", "status", "nodes")] + \
+               [("has_front", C.c_int32), ("has_back", C.c_int32)]
+
+
+class AdmmStep(C.Structure):       # hvp_admm_step
+    _fields_ = [("n", C.c_int32), ("N", C.c_int32), ("S", C.c_int32), ("phase", C.c_int32), ("nroles", C.c_int32),
+                ("leader_per_scenario", C.c_int32), ("leader_len", C.c_int64), ("T", C.c_int64), ("rho", C.c_double),
+                ("n_modes", C.c_int32), ("reserved", C.c_int32), ("mode_gear", C.c_int32 * 16),
+                ("role", AdmmStepRole * 4), ("role_of", C.c_int32 * 64)] + \
+               [(k, C.c_void_p) for k in ("t", "r", "x", "leader_x", "y_front", "y_back", "zf", "zb", "xs", "ND",
+                                          "failed_at", "u0", "gear0", "U_log", "ST")]
+
+
 CENT_PACK, CENT_ADOPT = 0, 1
 EVENT_PACK, EVENT_SELECT, EVENT_ADOPT = 0, 1, 2
+ADMM_PACK, ADMM_ROUND, ADMM_ADOPT = 0, 1, 2
 MPC_CENT, MPC_LOCAL, MPC_EVENT, MPC_ADMM, MPC_GADMM = 1, 2, 3, 4, 5
 MODEL_PWA_GEAR, MODEL_FRICTION_GEAR = 0, 1
 REAL_VEHICLE_REF, NO_LEADER = 8, -100
@@ -150,6 +165,7 @@ def lib():
     L.hvp_admm_round_dev.argtypes = [_vp, C.POINTER(AdmmRound), _vp]
     L.hvp_cent_step_dev.argtypes = [_vp, C.POINTER(CentStep), _vp]
     L.hvp_event_iter_dev.argtypes = [_vp, C.POINTER(EventIter), _vp]
+    L.hvp_admm_step_dev.argtypes = [_vp, C.POINTER(AdmmStep), _vp]
     L.hvp_microbench_fp64.argtypes = [_vp, C.c_int, C.POINTER(C.c_double)]
     L.hvp_microbench_smem.argtypes = [_vp, C.c_int, C.POINTER(C.c_double)]
     _lib = L

@@ -247,3 +247,12 @@ def event_iter_device(g, *, phase: int, ctx=None, stream=None):
     ctx = ctx or default_context()
     g.phase = int(phase)
     check(lib().hvp_event_iter_dev(ctx.handle, C.byref(g), _stream_arg(stream)))
+
+
+def admm_step_device(g, *, phase: int, ctx=None, stream=None):
+    """Fused glue of a naive-ADMM timestep (hvp_admm_step_dev): phase _lib.ADMM_PACK fills the role solves' inputs at the
+    start of a timestep, _lib.ADMM_ROUND does a round's z / y update, next parameters and logs, _lib.ADMM_ADOPT takes the
+    last round's first inputs and gears and logs them; `g` is a _lib.AdmmStep."""
+    ctx = ctx or default_context()
+    g.phase = int(phase)
+    check(lib().hvp_admm_step_dev(ctx.handle, C.byref(g), _stream_arg(stream)))

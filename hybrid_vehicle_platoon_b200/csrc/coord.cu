@@ -225,69 +225,161 @@ decent_observe_kernel(const __grid_constant__ ObsArgs A) {
 
 // ---- naive ADMM: z- and y-update of a consensus round and the next round's parameter vectors
 // (fleet_naive_admm.py:421-468) in one launch, read straight from the role solves' outputs -------------------------------
+// The same device code serves hvp_admm_round_dev (step = false: leader window from lwin, no statuses, no logs) and the
+// three phases of hvp_admm_step_dev (step = true: t / r on the device, leader window from the trajectory, zeros for a
+// solve that was not optimal, logs).
 struct ARole {
     double* params;                   // [count*S][5 * 2(N+1)]: leader window | y_front | z_front | y_back | z_back
+    double* x0;                       // [count*S][1][2]     (step PACK)
     const double* xo;                 // [count*S][2][N+1]   own prediction of the round just solved
     const double* eo;                 // [count*S][ne]       copies: x_front (if not front) then x_back (if not trailer)
+    const double* u;                  // [count*S][N]        (step ADOPT)
+    const int32_t *modes, *status, *nodes;   // step only; status NULL: every solve counts as optimal
     int count, ne, has_front, has_back;
 };
 struct AdmmArgs {
-    int n, N, S, nroles, pack_only;
+    int n, N, S, nroles, phase;       // phase: HVP_ADMM_PACK | HVP_ADMM_ROUND | HVP_ADMM_ADOPT
+    bool step;
     double rho;
     ARole role[4];
     int role_of[64], local_of[64];    // vehicle -> role, index among the role's vehicles
-    const double* lwin;               // [S][2][N+1]
+    const double* lwin;               // hvp_admm_round_dev: [S][2][N+1]
+    const long long* t;               // step: device timestep index
+    const int32_t* r;                 // step: device round index
+    const double *x, *lx;             // step: states [S][n][2], leader trajectory [S or 1][2][lx_len]
+    long long lx_len, lx_sstride, T;
+    int n_modes;
+    int mode_gear[16];
     double *y_front, *y_back, *zf, *zb, *xs;   // [S][n][2][N+1] each
+    int32_t *ND, *fa, *gear0, *ST;
+    double *u0, *U;
 };
-struct AOut { const double *own, *cf, *cb; };
+__device__ __forceinline__ int64_t arow(const AdmmArgs& A, int s, int j) {
+    return (int64_t)s * A.role[A.role_of[j]].count + A.local_of[j];
+}
+__device__ __forceinline__ bool aok(const ARole& R, int64_t b) { return !R.status || R.status[b] == HVP_OPTIMAL; }
+// what vehicle j's solve contributes to the z-update: its own prediction and the copies it holds of its neighbours,
+// all zero when the solve was not optimal (solve_mpc(raises=False) zeros x and the copies, LocalMpcADMM._post)
+struct AOut { const double *own, *cf, *cb; bool ok; };
 __device__ __forceinline__ AOut aout(const AdmmArgs& A, int s, int j) {
+    AOut o = {nullptr, nullptr, nullptr, false};
+    if (j < 0 || j >= A.n) return o;
     const ARole& R = A.role[A.role_of[j]];
-    const int64_t b = (int64_t)s * R.count + A.local_of[j];
+    const int64_t b = arow(A, s, j);
     const int blk = 2 * (A.N + 1);
-    AOut o;
     o.own = R.xo + b * blk;
     const double* e = R.eo + b * R.ne;
     o.cf = R.has_front ? e : nullptr;
     o.cb = R.has_back ? e + (R.has_front ? blk : 0) : nullptr;
+    o.ok = aok(R, b);
     return o;
 }
-// z of vehicle j: (own + x_front copy held by j+1) / 2 at the front, (own + x_back copy held by j-1) / 2 at the rear,
-// (own + both) / 3 inside -- in exactly this order of additions (fleet_naive_admm.py:421-447)
-__device__ __forceinline__ double azval(const AdmmArgs& A, int s, int j, int e) {
-    const double own = aout(A, s, j).own[e];
-    if (j == 0) return __dadd_rn(own, aout(A, s, 1).cf[e]) / 2.0;
-    if (j == A.n - 1) return __dadd_rn(own, aout(A, s, j - 1).cb[e]) / 2.0;
-    return __dadd_rn(__dadd_rn(own, aout(A, s, j + 1).cf[e]), aout(A, s, j - 1).cb[e]) / 3.0;
+__device__ __forceinline__ double aval(const double* p, bool ok, int e) { return ok ? p[e] : 0.0; }
+// z of vehicle k (a, m, b: the outputs of vehicles k-1, k, k+1): (own + x_front copy held by k+1) / 2 at the front,
+// (own + x_back copy held by k-1) / 2 at the rear, (own + both) / 3 inside -- in exactly this order of additions
+// (fleet_naive_admm.py:421-447)
+__device__ __forceinline__ double azval(int n, int k, const AOut& a, const AOut& m, const AOut& b, int e) {
+    const double own = aval(m.own, m.ok, e);
+    if (k == 0) return __dadd_rn(own, aval(b.cf, b.ok, e)) / 2.0;
+    if (k == n - 1) return __dadd_rn(own, aval(a.cb, a.ok, e)) / 2.0;
+    return __dadd_rn(__dadd_rn(own, aval(b.cf, b.ok, e)), aval(a.cb, a.ok, e)) / 3.0;
+}
+// entry e of the leader-window block: lwin, or leader_x[:, t : t+N+1] with columns past the end reading the last one
+__device__ __forceinline__ double alwin(const AdmmArgs& A, int s, int e, long long t) {
+    const int np1 = A.N + 1;
+    if (!A.step) return A.lwin[(size_t)s * 2 * np1 + e];
+    const int row = e / np1;
+    long long c = t + (e - row * np1);
+    c = c < 0 ? 0 : (c >= A.lx_len ? A.lx_len - 1 : c);
+    return A.lx[(size_t)s * A.lx_sstride + row * A.lx_len + c];
 }
 __global__ void __launch_bounds__(128)
 admm_round_kernel(const __grid_constant__ AdmmArgs A) {
     const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int n = A.n, blk = 2 * (A.N + 1);
+    const int n = A.n, N = A.N, np1 = N + 1, blk = 2 * np1;
     if (tid >= (int64_t)A.S * n) return;
     const int s = (int)(tid / n), j = (int)(tid - (int64_t)s * n);
-    const AOut me = aout(A, s, j);
     const ARole& R = A.role[A.role_of[j]];
-    double* P = R.params + ((size_t)s * R.count + A.local_of[j]) * (5 * blk);
+    const int64_t b = arow(A, s, j);
+    const long long t = A.step ? *A.t : 0;
+    if (A.phase == HVP_ADMM_ADOPT) {  // first inputs of the last round, gears from the mode table, logs
+        const bool ok = aok(R, b);
+        const double u0 = ok ? R.u[b * N] : 0.0;
+        A.u0[tid] = u0;
+        int gear = 6;
+        if (A.gear0) {
+            if (ok) {
+                int m = R.modes[b * N];
+                m = m < 0 ? 0 : (m >= A.n_modes ? A.n_modes - 1 : m);
+                gear = A.mode_gear[m];
+            }
+            A.gear0[tid] = gear;
+        }
+        if (t < 0 || t >= A.T) return;
+        const size_t row = (size_t)t * A.S + s;
+        double* Ur = A.U + row * (A.gear0 ? 2 * n : n);
+        Ur[j] = u0;
+        if (A.gear0) Ur[n + j] = (double)gear;
+        A.ST[row * n + j] = R.status[b];
+        return;
+    }
+    double* P = R.params + b * (5 * blk);
     const size_t o = (size_t)tid * blk;
-    const double* lw = A.lwin + (size_t)s * blk;
+    if (A.phase == HVP_ADMM_PACK) {
+        if (A.step) {
+            R.x0[2 * b] = A.x[2 * tid]; R.x0[2 * b + 1] = A.x[2 * tid + 1];
+            if (t > 0) {              // the neighbours' previous predictions, shifted (fleet_naive_admm.py:392-402)
+                for (int e = 0; e < blk; ++e) {
+                    const int row = e / np1, k = e - row * np1, src = row * np1 + (k < N ? k + 1 : N);
+                    if (j > 0) A.zf[o + e] = A.xs[o - blk + src];
+                    if (j < n - 1) A.zb[o + e] = A.xs[o + blk + src];
+                }
+            }
+        }
+        for (int e = 0; e < blk; ++e) {
+            P[e] = alwin(A, s, e, t); P[blk + e] = A.y_front[o + e]; P[2 * blk + e] = A.zf[o + e];
+            P[3 * blk + e] = A.y_back[o + e]; P[4 * blk + e] = A.zb[o + e];
+        }
+        return;
+    }
+    AOut w[5];                        // vehicles j-2 .. j+2
+    for (int d = 0; d < 5; ++d) w[d] = aout(A, s, j - 2 + d);
+    const AOut& me = w[2];
     for (int e = 0; e < blk; ++e) {
         double yf = A.y_front[o + e], yb = A.y_back[o + e], zfv = A.zf[o + e], zbv = A.zb[o + e];
-        if (A.pack_only) {
-            P[e] = lw[e]; P[blk + e] = yf; P[2 * blk + e] = zfv; P[3 * blk + e] = yb; P[4 * blk + e] = zbv;
-            continue;
-        }
-        A.xs[o + e] = me.own[e];
+        A.xs[o + e] = aval(me.own, me.ok, e);
         if (j > 0) {                  // y_front += rho (x_front copy - z of the vehicle in front); next target z_{j-1}
-            zfv = azval(A, s, j - 1, e);
-            yf = __dadd_rn(yf, __dmul_rn(A.rho, __dadd_rn(me.cf[e], -zfv)));
+            zfv = azval(n, j - 1, w[0], w[1], w[2], e);
+            yf = __dadd_rn(yf, __dmul_rn(A.rho, __dadd_rn(aval(me.cf, me.ok, e), -zfv)));
         }
         if (j < n - 1) {
-            zbv = azval(A, s, j + 1, e);
-            yb = __dadd_rn(yb, __dmul_rn(A.rho, __dadd_rn(me.cb[e], -zbv)));
+            zbv = azval(n, j + 1, w[2], w[3], w[4], e);
+            yb = __dadd_rn(yb, __dmul_rn(A.rho, __dadd_rn(aval(me.cb, me.ok, e), -zbv)));
         }
         A.y_front[o + e] = yf; A.y_back[o + e] = yb; A.zf[o + e] = zfv; A.zb[o + e] = zbv;
-        P[e] = lw[e]; P[blk + e] = yf; P[2 * blk + e] = zfv; P[3 * blk + e] = yb; P[4 * blk + e] = zbv;
+        P[e] = alwin(A, s, e, t); P[blk + e] = yf; P[2 * blk + e] = zfv; P[3 * blk + e] = yb; P[4 * blk + e] = zbv;
     }
+    // logs of the round.  ND: every vehicle's node count (a max: the same whatever the order).  failed_at: in the first
+    // round of the episode the scenario's first thread resets the row and scans every vehicle; later, only a vehicle whose
+    // solve failed looks at the vehicles before it, and the lowest failing one writes the row if it is still empty -- one
+    // writer per scenario, and nothing beyond the atomic for the rounds in which every solve is optimal
+    if (!A.step || t < 0 || t >= A.T) return;
+    const int rr = *A.r;
+    atomicMax(A.ND + (size_t)t * A.S + s, R.nodes[b]);
+    int32_t* F = A.fa + 3 * (size_t)s;
+    if (t == 0 && rr == 0) {
+        if (j != 0) return;
+        F[0] = -1; F[1] = -1; F[2] = 0;
+        for (int i = 0; i < n; ++i) {
+            const int st = A.role[A.role_of[i]].status[arow(A, s, i)];
+            if (st != HVP_OPTIMAL) { F[0] = 0; F[1] = 0; F[2] = st; break; }
+        }
+        return;
+    }
+    if (me.ok) return;
+    for (int i = 0; i < j; ++i)
+        if (A.role[A.role_of[i]].status[arow(A, s, i)] != HVP_OPTIMAL) return;
+    if (F[0] < 0) { F[0] = (int32_t)t; F[1] = rr; F[2] = R.status[b]; }
 }
 
 // ---- centralized controller: the leader window before the solve, the adoption of its answer after it
@@ -561,8 +653,9 @@ extern "C" int hvp_admm_round_dev(hvp_ctx* c, const hvp_admm_round* g, void* str
         return hvp_fail(-4, "admm_round: bad sizes (n=%d N=%d S=%d roles=%d)", g->n, g->N, g->S, g->nroles);
     if (g->S == 0) return 0;
     if (!g->lwin || !g->y_front || !g->y_back || !g->zf || !g->zb || !g->xs) return hvp_fail(-1, "admm_round: NULL array argument");
-    AdmmArgs A;
-    A.n = g->n; A.N = g->N; A.S = g->S; A.nroles = g->nroles; A.rho = g->rho; A.pack_only = g->pack_only;
+    AdmmArgs A = {};
+    A.n = g->n; A.N = g->N; A.S = g->S; A.nroles = g->nroles; A.rho = g->rho;
+    A.phase = g->pack_only ? HVP_ADMM_PACK : HVP_ADMM_ROUND;
     const int blk = 2 * (g->N + 1);
     int counts[4] = {0, 0, 0, 0};
     for (int i = 0; i < g->n; ++i) {
@@ -591,6 +684,69 @@ extern "C" int hvp_admm_round_dev(hvp_ctx* c, const hvp_admm_round* g, void* str
     admm_round_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(A);
     e = cudaGetLastError();
     if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "admm_round: launch failed: %s", cudaGetErrorString(e));
+    c->launches += 1;
+    return 0;
+}
+
+// hvp.h: hvp_admm_step_dev
+extern "C" int hvp_admm_step_dev(hvp_ctx* c, const hvp_admm_step* g, void* stream) {
+    if (!c || !g) return hvp_fail(-1, "admm_step: NULL argument");
+    const int n = g->n, ph = g->phase;
+    if (n < 2 || n > 64 || g->N < 1 || g->S < 0 || g->nroles < 1 || g->nroles > 4 || g->T < 0 ||
+        (ph != HVP_ADMM_PACK && ph != HVP_ADMM_ROUND && ph != HVP_ADMM_ADOPT))
+        return hvp_fail(-4, "admm_step: bad sizes (n=%d N=%d S=%d roles=%d T=%lld phase=%d)", n, g->N, g->S, g->nroles,
+                        (long long)g->T, ph);
+    if ((ph != HVP_ADMM_ADOPT && g->leader_len < 1) || (ph == HVP_ADMM_ADOPT && g->gear0 && (g->n_modes < 1 || g->n_modes > 16)))
+        return hvp_fail(-4, "admm_step: bad sizes (leader_len=%lld n_modes=%d)", (long long)g->leader_len, g->n_modes);
+    AdmmArgs A = {};
+    A.n = n; A.N = g->N; A.S = g->S; A.nroles = g->nroles; A.rho = g->rho; A.phase = ph; A.step = true;
+    const int blk = 2 * (g->N + 1);
+    int counts[4] = {0, 0, 0, 0};
+    for (int i = 0; i < n; ++i) {
+        const int r = g->role_of[i];
+        if (r < 0 || r >= g->nroles) return hvp_fail(-4, "admm_step: role_of[%d] = %d out of range", i, r);
+        A.role_of[i] = r; A.local_of[i] = counts[r]++;
+    }
+    for (int r = 0; r < g->nroles; ++r) {
+        const hvp_admm_step_role& s = g->role[r];
+        ARole& R = A.role[r];
+        R.params = s.params; R.x0 = s.x0; R.xo = s.x; R.eo = s.extra; R.u = s.u; R.modes = s.modes; R.status = s.status;
+        R.nodes = s.nodes; R.count = counts[r];
+        R.has_front = s.has_front; R.has_back = s.has_back; R.ne = (s.has_front + s.has_back) * blk;
+    }
+    // a vehicle reads the copies its neighbours hold of it: vehicle i > 0 must hold x_front, i < n-1 must hold x_back
+    for (int i = 0; i < n; ++i) {
+        const ARole& R = A.role[A.role_of[i]];
+        if ((i > 0) != (R.has_front != 0) || (i < n - 1) != (R.has_back != 0))
+            return hvp_fail(-4, "admm_step: role of vehicle %d does not match its position (front / trailer copies)", i);
+    }
+    if (g->S == 0) return 0;
+    if (!g->t || !g->y_front || !g->y_back || !g->zf || !g->zb || !g->xs ||
+        (ph == HVP_ADMM_PACK && (!g->x || !g->leader_x)) ||
+        (ph == HVP_ADMM_ROUND && (!g->r || !g->leader_x || !g->ND || !g->failed_at)) ||
+        (ph == HVP_ADMM_ADOPT && (!g->u0 || !g->U_log || !g->ST)))
+        return hvp_fail(-1, "admm_step: NULL array argument (phase %d)", ph);
+    for (int r = 0; r < g->nroles; ++r) {
+        const ARole& R = A.role[r];
+        if (R.count == 0) continue;
+        if ((ph == HVP_ADMM_PACK && (!R.params || !R.x0)) ||
+            (ph == HVP_ADMM_ROUND && (!R.params || !R.xo || (R.ne > 0 && !R.eo) || !R.status || !R.nodes)) ||
+            (ph == HVP_ADMM_ADOPT && (!R.u || !R.status || (g->gear0 && !R.modes))))
+            return hvp_fail(-1, "admm_step: NULL role buffer (role %d, phase %d)", r, ph);
+    }
+    A.t = (const long long*)g->t; A.r = g->r; A.x = g->x; A.lx = g->leader_x;
+    A.lx_len = g->leader_len; A.lx_sstride = g->leader_per_scenario ? 2 * g->leader_len : 0; A.T = g->T;
+    A.n_modes = g->n_modes;
+    for (int m = 0; m < 16; ++m) A.mode_gear[m] = g->mode_gear[m];
+    A.y_front = g->y_front; A.y_back = g->y_back; A.zf = g->zf; A.zb = g->zb; A.xs = g->xs;
+    A.ND = g->ND; A.fa = g->failed_at; A.u0 = g->u0; A.gear0 = g->gear0; A.U = g->U_log; A.ST = g->ST;
+    cudaError_t e = cudaSetDevice(c->device);
+    if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "admm_step: cudaSetDevice: %s", cudaGetErrorString(e));
+    cudaStream_t st = stream ? (cudaStream_t)stream : c->stream;
+    const int64_t threads = (int64_t)g->S * n;
+    admm_round_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(A);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return hvp_fail(-100 - (int)e, "admm_step: launch failed: %s", cudaGetErrorString(e));
     c->launches += 1;
     return 0;
 }

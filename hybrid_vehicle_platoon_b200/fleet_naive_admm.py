@@ -6,7 +6,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from ._sim import collect, make_env_and_systems
+from ._sim import collect, make_env_and_systems, save_results
 from .agents import MldAgent
 from .misc import Params, Sim
 from .mpc import LocalMpcADMM, solve_compiled_batch
@@ -101,3 +101,63 @@ def simulate(sim: Sim, admm_iters: int = 20, save: bool = False, plot: bool = Fa
                             ep_len=ep_len, N=N, leader_x=leader_x, ts=ts)
     agent.evaluate(env=env, episodes=1, seed=seed)
     return collect(env, agent, leader_x, f"admm_{admm_iters}_{sim.id}_seed_{seed}.pkl", save)
+
+
+def simulate_many(sim: Sim, seeds, admm_iters: int = 20, leader_index: int = 0, ep_len=None, save: bool = False,
+                  strict: bool = True, ctx=None):
+    """simulate() for several seeds of one configuration in ONE on-device closed loop (sweep.BatchedAdmmSweep): the
+    paper's "10 seeds of a configuration" in one call.  Each seed's initial state is PlatoonEnv.reset with the seed
+    MldAgent.evaluate derives from it, the masses and d_safe are the env's, rho is 0.5 and the solver options are the
+    ones simulate() would use (mpc.OPTIONS); sim.real_vehicle_as_reference goes to the rollout as simulate() gives it to
+    PlatoonEnv.  Every Sim simulate() accepts is accepted (this controller ignores open_loop and quadratic_cost), except
+    n < 2: the batched loop needs at least two vehicles.  Returns one dict per seed with simulate()'s 7 objects and
+    shapes, except solve_times, which is NaN: a batched launch has no per-scenario solve time; node_counts is the
+    largest node count over the rounds and vehicles of a timestep.  save=True writes simulate()'s pickle per seed.
+    strict=True raises what simulate() would after the run, naming the seed and timestep: RuntimeError("Infeasible
+    problem encountered ...") for a solve that was not optimal (RuntimeWarning with pwa_friction, as the gear MPC
+    raises), the rollout's error otherwise, whichever comes first in the episode; strict=False returns the episodes as
+    computed, with a vehicle whose solve was not optimal applying zero input (gear 6), as solve_mpc(raises=False)."""
+    from .env import raise_rollout_error
+    from .mpc import OPTIONS
+    from .sweep import BatchedAdmmSweep
+    n, N = sim.n, sim.N
+    if n < 2:
+        raise ValueError("the batched ADMM loop needs at least two vehicles")
+    seeds = [int(s) for s in seeds]
+    leader_x = sim.leader_trajectory.get_leader_trajectory()
+    env, _, _, ep_len = make_env_and_systems(sim, leader_index, ep_len, None)
+    base = env.unwrapped
+    x0 = np.stack([np.asarray(env.reset(seed=int(np.random.SeedSequence(s).generate_state(1)[0]))[0],
+                              dtype=np.float64).reshape(2 * n) for s in seeds])
+    sw = BatchedAdmmSweep(n, N, admm_iters=admm_iters, rho=0.5, masses=base.masses, spacing_policy=sim.spacing_policy,
+                          leader_index=leader_index, d_safe=base.d_safe, model=sim.vehicle_model_type,
+                          mip_gap=OPTIONS.mip_gap, time_limit_ms=OPTIONS.time_limit * 1e3,
+                          real_vehicle_as_reference=sim.real_vehicle_as_reference, ctx=ctx)
+    try:
+        r = sw.run(x0, leader_x, ep_len)
+    finally:
+        sw.close()
+    if strict:
+        # what simulate() meets first in each episode; the first episode (in seed order) that meets one is reported
+        for j, seed in enumerate(seeds):
+            bad_t, _, st = (int(v) for v in r["failed_at"][j])
+            err_t = np.nonzero(r["errors"][:, j])[0]
+            if bad_t >= 0 and (not err_t.size or bad_t <= err_t[0]):
+                if sim.vehicle_model_type == "pwa_friction":      # mpcs/mpc_gear.py:127-128
+                    raise RuntimeWarning(f"gear mpc is infeasible (status {st}; seed {seed}, timestep {bad_t})")
+                raise RuntimeError(f"Infeasible problem encountered (status {st}). (seed {seed}, timestep {bad_t})")
+            if err_t.size:
+                try:
+                    raise_rollout_error(int(r["errors"][err_t[0], j]))
+                except RuntimeError as e:
+                    raise RuntimeError(f"{e} (seed {seed}, timestep {int(err_t[0])})") from None
+    out = []
+    for j, seed in enumerate(seeds):
+        # shapes of collect(): X (T+1,2n), U (T,n|2n), R (T,1,1), solve_times / node_counts (T,1), violations (T,)
+        res = dict(X=r["X"][:, j].copy(), U=r["U"][:, j].copy(), R=r["R"][:, j].reshape(ep_len, 1, 1).copy(),
+                   solve_times=np.full((ep_len, 1), np.nan), node_counts=r["nodes"][:, j].astype(np.float64).reshape(ep_len, 1),
+                   violations=np.where(r["violations"][:, j] != 0, 100.0, 0.0), leader_x=leader_x)
+        if save:
+            save_results(res, f"admm_{admm_iters}_{sim.id}_seed_{seed}.pkl")
+        out.append(res)
+    return out

@@ -525,21 +525,40 @@ class BatchedAdmmSweep:
     """S independent platoons under the naive (non-convex) ADMM controller (fleet_naive_admm.py:320-587), all
     state on the device.  One timestep = admm_iters rounds; one round = the x-update of all S*n vehicles (one launch
     of the compiled-MPC kernel per distinct role: front / interior / trailer, leader where applicable) followed by
-    the z- and y-updates as a few torch ops over (S, n, 2, N+1) tensors; then one rollout launch."""
+    the z- and y-updates; then one rollout launch.  A vehicle whose solve is not optimal contributes zeros for its
+    prediction and its copies and applies zero input (gear 6), as solve_mpc(raises=False) gives it.
+
+    model: "pwa_gear" (gears derived from the velocities) or "pwa_friction" (discrete gears chosen by the MPC; the
+    action is [u_g ; gears]).  mip_gap / time_limit_ms: the role solves' options (mpc.OPTIONS in simulate()).
+    real_vehicle_as_reference: the rollout's stage cost tracks the real vehicle in front (PlatoonEnv's option).
+    fused: the glue of a timestep as the three phases of ONE kernel (hvp_admm_step_dev, csrc/coord.cu) with the
+    timestep and round indices on the device; None reads HVP_SWEEP_FUSED (default on).  fused=False keeps the glue as
+    torch ops indexed by the host loop, pwa_gear only: the reference the kernel is tested against.
+    fork: the roles' solves on forked streams; graph (fused loop): each round replayed as a CUDA graph."""
 
     def __init__(self, n: int, N: int, admm_iters: int = 20, rho: float = 0.5, masses=None,
                  spacing_policy=ConstantSpacingPolicy(50), leader_index: int = 0, d_safe: float = Params.d_safe,
-                 device: int = 0, ctx=None, graph: bool = False, fork: bool = True, fused=None):
+                 model: str = "pwa_gear", mip_gap: float = 0.0, time_limit_ms: float = 0.0,
+                 real_vehicle_as_reference: bool = False, device: int = 0, ctx=None, graph: bool = False,
+                 fork: bool = True, fused=None):
         import os
         import torch
-        from ._lib import MPC_ADMM
+        from ._lib import MODEL_FRICTION_GEAR, MODEL_PWA_GEAR, MPC_ADMM
         self.graph, self.fork = graph, fork
-        # fused: z / y update and parameter packing of a round as one CUDA kernel (csrc/coord.cu hvp_admm_round_dev);
-        # False keeps them as torch ops (the reference the kernel is tested against)
+        if model not in ("pwa_gear", "pwa_friction"):
+            raise ValueError(f"model must be 'pwa_gear' or 'pwa_friction', got {model!r}")
         self.fused = (os.environ.get("HVP_SWEEP_FUSED", "1") != "0") if fused is None else bool(fused)
+        self.friction = model == "pwa_friction"
+        if self.friction and not self.fused:
+            raise ValueError("the torch glue (fused=False) runs the pwa_gear model only")
         if n < 2:
             raise ValueError("the ADMM scheme needs at least two vehicles")
+        if self.fused and (n > 64 or admm_iters < 1):
+            raise ValueError(f"the fused loop needs n <= 64 and admm_iters >= 1 (n = {n}, admm_iters = {admm_iters})")
+        if leader_index != 0 and real_vehicle_as_reference:
+            raise NotImplementedError("Not implemented for real vehicle with leader not 0.")   # as PlatoonEnv
         self.torch, self.n, self.N, self.iters, self.rho, self.leader_index = torch, n, N, admm_iters, rho, leader_index
+        self.real_ref = bool(real_vehicle_as_reference)
         self.dev = torch.device("cuda", device)
         self.ctx = ctx or default_context(device)
         self.d0, self.t0 = spacing_params(spacing_policy)
@@ -551,151 +570,227 @@ class BatchedAdmmSweep:
         for i in range(n):
             fl = (FRONT if i == 0 else 0) | (TRAILER if i == n - 1 else 0) | (LEADER if i == leader_index else 0)
             if fl not in roles:
-                roles[fl] = api.CompiledMpc(MPC_ADMM, N, flags=fl, rho=rho, d0=self.d0, t0=self.t0, ctx=self.ctx)
+                roles[fl] = api.CompiledMpc(MPC_ADMM, N, model=MODEL_FRICTION_GEAR if self.friction else MODEL_PWA_GEAR,
+                                            flags=fl, rho=rho, d0=self.d0, t0=self.t0, mip_gap=mip_gap,
+                                            time_limit_ms=time_limit_ms, ctx=self.ctx)
             self.role_of.append(fl)
         self.roles = roles
 
+    def close(self):
+        """Releases the compiled formulations (their device scratch)."""
+        for cm in self.roles.values():
+            cm.close()
+        self.roles = {}
+
     def run(self, x0, leader_x, ep_len: int):
-        """Same contract as BatchedDecentSweep.run; additionally returns nothing about the consensus variables."""
-        torch, dev, n, N, rho = self.torch, self.dev, self.n, self.N, self.rho
-        f64, np1 = torch.float64, N + 1
-        x = torch.as_tensor(np.ascontiguousarray(x0, dtype=np.float64), device=dev)
-        S = x.shape[0]
-        lx = torch.as_tensor(np.ascontiguousarray(leader_x, dtype=np.float64), device=dev)
-        if lx.ndim == 2:
-            lx = lx.unsqueeze(0).expand(S, -1, -1)
+        """x0 (S,2n) initial states, leader_x (2,>=ep_len+N) shared or (S,2,>=ep_len+N) per scenario.  Returns dict of
+        numpy arrays: X (T+1,S,2n), U (T,S,n) -- (T,S,2n) = [u_g ; gears] for pwa_friction --, R (T,S), violations (T,S)
+        uint8, errors (T,S) int32, status (T,S,n) int32 of the last round, nodes (T,S) int32 (max over the rounds and
+        vehicles of a timestep) and failed_at (S,3) int32: (timestep, round, status) of the first solve that was not
+        optimal -- the lowest vehicle index within the first such round -- or (-1, -1, 0)."""
+        torch, dev, n, N = self.torch, self.dev, self.n, self.N
+        f64, i32, np1 = torch.float64, torch.int32, N + 1
+        if not self.roles:
+            raise RuntimeError("BatchedAdmmSweep is closed")
+        x0 = np.ascontiguousarray(x0, dtype=np.float64)
+        if x0.ndim != 2 or x0.shape[1] != 2 * n:
+            raise ValueError(f"x0 must have shape (S, {2 * n}), got {x0.shape}")
+        S, T = x0.shape[0], int(ep_len)
+        lx_np = np.ascontiguousarray(leader_x, dtype=np.float64)
+        if lx_np.ndim not in (2, 3) or lx_np.shape[-2] != 2 or (lx_np.ndim == 3 and lx_np.shape[0] != S):
+            raise ValueError(f"leader_x must have shape (2, L) or ({S}, 2, L), got {lx_np.shape}")
+        if lx_np.shape[-1] < T + N:
+            raise ValueError("leader trajectory shorter than ep_len + N")
+        x = torch.as_tensor(x0, device=dev)
+        lx = torch.as_tensor(lx_np, device=dev)
         m = np.full((S, n), 800.0) if self.masses is None else np.broadcast_to(self.masses, (S, n))
         d_mass = torch.as_tensor(np.array(m, dtype=np.float64, order="C"), device=dev)
-        edesc = api.env_desc(n, self.leader_index, self.d0, self.t0, self.d_safe, True, False, True)
+        edesc = api.env_desc(n, self.leader_index, self.d0, self.t0, self.d_safe, True, self.real_ref, True)
         zeros = lambda *s: torch.zeros(s, dtype=f64, device=dev)
-        y_front, y_back, z = zeros(S, n, 2, np1), zeros(S, n, 2, np1), zeros(S, n, 2, np1)
-        zf, zb = zeros(S, n, 2, np1), zeros(S, n, 2, np1)        # the z each vehicle's copies are pulled towards
-        xs = zeros(S, n, 2, np1)                                  # own predictions of the last round
-        cf, cb = zeros(S, n, 2, np1), zeros(S, n, 2, np1)        # copies x_front / x_back of the last round
-        have_pred = False
-        # per-role gather indices and work buffers
+        # consensus variables [S][n][2][N+1]: multipliers, the z each vehicle's copies are pulled towards, own predictions
+        cons = dict(y_front=zeros(S, n, 2, np1), y_back=zeros(S, n, 2, np1), zf=zeros(S, n, 2, np1),
+                    zb=zeros(S, n, 2, np1), xs=zeros(S, n, 2, np1))
+        # per-role solve buffers, rows [scenario][vehicle of the role]
         groups = {}
         for fl, cm in self.roles.items():
-            idx = torch.as_tensor([i for i in range(n) if self.role_of[i] == fl], device=dev)
+            idx = [i for i in range(n) if self.role_of[i] == fl]
             k = len(idx); B = S * k
-            groups[fl] = dict(cm=cm, idx=idx, k=k, B=B,
+            groups[fl] = dict(cm=cm, idx=torch.as_tensor(idx, device=dev), k=k, B=B,
+                              m=d_mass[:, idx].reshape(B, 1).contiguous(),
                               u=torch.empty((B, 1, N), dtype=f64, device=dev), x=torch.empty((B, 1, 2, np1), dtype=f64, device=dev),
                               e=torch.empty((B, max(cm.n_extra, 1)), dtype=f64, device=dev),
-                              mo=torch.empty((B, 1, N), dtype=torch.int32, device=dev), ob=torch.empty(B, dtype=f64, device=dev),
-                              st=torch.empty(B, dtype=torch.int32, device=dev), no=torch.empty(B, dtype=torch.int32, device=dev))
-        X = torch.empty((ep_len + 1, S, 2 * n), dtype=f64, device=dev)
-        U = torch.empty((ep_len, S, n), dtype=f64, device=dev)
-        R = torch.empty((ep_len, S), dtype=f64, device=dev)
-        V = torch.empty((ep_len, S), dtype=torch.uint8, device=dev)
-        E = torch.empty((ep_len, S), dtype=torch.int32, device=dev)
-        ST = torch.empty((ep_len, S, n), dtype=torch.int32, device=dev)
+                              mo=torch.empty((B, 1, N), dtype=i32, device=dev), ob=torch.empty(B, dtype=f64, device=dev),
+                              st=torch.empty(B, dtype=i32, device=dev), no=torch.empty(B, dtype=i32, device=dev))
+        X = torch.empty((T + 1, S, 2 * n), dtype=f64, device=dev)
+        U = torch.empty((T, S, 2 * n if self.friction else n), dtype=f64, device=dev)
+        R = torch.empty((T, S), dtype=f64, device=dev)
+        V = torch.empty((T, S), dtype=torch.uint8, device=dev)
+        E = torch.empty((T, S), dtype=i32, device=dev)
+        ST = torch.empty((T, S, n), dtype=i32, device=dev)
+        ND = torch.zeros((T, S), dtype=i32, device=dev)
+        FA = torch.tensor([[-1, -1, 0]] * S, dtype=i32, device=dev).reshape(S, 3)
         X[0] = x
-        u0 = torch.empty((S, n), dtype=f64, device=dev)
-        stat = torch.empty((S, n), dtype=torch.int32, device=dev)
-        x_cur = x.clone()                                         # state the rounds of this timestep start from (static)
-        lwin = torch.empty((S, 1, 2 * np1), dtype=f64, device=dev)
-        three = torch.full((), 3.0, dtype=f64, device=dev)
-
-        def role_piece(fl, g):
-            def piece():
-                stream = torch.cuda.current_stream().cuda_stream
-                idx, k, B = g["idx"], g["k"], g["B"]
-                params = torch.cat((lwin.expand(S, k, -1), y_front[:, idx].reshape(S, k, -1), zf[:, idx].reshape(S, k, -1),
-                                    y_back[:, idx].reshape(S, k, -1), zb[:, idx].reshape(S, k, -1)), dim=2).reshape(B, -1).contiguous()
-                x0g = x_cur.view(S, n, 2)[:, idx].reshape(B, 1, 2).contiguous()
-                mg = d_mass[:, idx].reshape(B, 1).contiguous()
-                g["cm"].solve_device(B, x0g, mg, params, None, g["u"], g["x"], g["e"], g["mo"], g["ob"], g["st"],
-                                     g["no"], None, stream=stream)
-                xs[:, idx] = g["x"].view(S, k, 2, np1)
-                u0[:, idx] = g["u"].view(S, k, N)[:, :, 0]
-                stat[:, idx] = g["st"].view(S, k)
-                e = g["e"].view(S, k, -1)
-                o = 0
-                if not fl & FRONT:
-                    cf[:, idx] = e[:, :, o:o + 2 * np1].reshape(S, k, 2, np1); o += 2 * np1
-                if not fl & TRAILER:
-                    cb[:, idx] = e[:, :, o:o + 2 * np1].reshape(S, k, 2, np1)
-            return piece
-
-        ar = None
+        logs = (X, U, R, V, E, ST, ND, FA)
         if self.fused:
-            from . import _lib
-            ar = _lib.AdmmRound()
-            ar.n, ar.N, ar.S, ar.nroles, ar.rho = n, N, S, len(groups), rho
-            order = list(groups)
-            for i in range(n):
-                ar.role_of[i] = order.index(self.role_of[i])
-            for r, fl in enumerate(order):
-                g = groups[fl]
-                g["params"] = torch.zeros((g["B"], g["cm"].n_param), dtype=f64, device=dev)
-                g["x0"] = torch.zeros((g["B"], 1, 2), dtype=f64, device=dev)
-                g["m"] = d_mass[:, g["idx"]].reshape(g["B"], 1).contiguous()
-                R_ = ar.role[r]
-                R_.params, R_.x, R_.extra = g["params"].data_ptr(), g["x"].data_ptr(), g["e"].data_ptr()
-                R_.has_front, R_.has_back = int(not fl & FRONT), int(not fl & TRAILER)
-            ar.lwin = lwin.data_ptr()
-            ar.y_front, ar.y_back, ar.zf, ar.zb, ar.xs = (t_.data_ptr() for t_ in (y_front, y_back, zf, zb, xs))
+            self._run_fused(S, T, x, lx, d_mass, edesc, cons, groups, logs)
+        else:
+            self._run_torch(S, T, x, lx, d_mass, edesc, cons, groups, logs)
+        torch.cuda.synchronize()
+        return dict(X=X.cpu().numpy(), U=U.cpu().numpy(), R=R.cpu().numpy(), violations=V.cpu().numpy(),
+                    errors=E.cpu().numpy(), status=ST.cpu().numpy(), nodes=ND.cpu().numpy(), failed_at=FA.cpu().numpy())
 
-            def fused_piece(g):
-                def piece():
-                    g["cm"].solve_device(g["B"], g["x0"], g["m"], g["params"], None, g["u"], g["x"], g["e"], g["mo"], g["ob"],
-                                         g["st"], g["no"], None, stream=torch.cuda.current_stream().cuda_stream)
-                return piece
-        pieces = [fused_piece(g) for g in groups.values()] if ar is not None else [role_piece(fl, g) for fl, g in groups.items()]
+    def _solve(self, g, x0, params):
+        stream = self.torch.cuda.current_stream().cuda_stream
+        g["cm"].solve_device(g["B"], x0, g["m"], params, None, g["u"], g["x"], g["e"], g["mo"], g["ob"], g["st"], g["no"],
+                             None, stream=stream)
+
+    def _run_fused(self, S, T, x, lx, d_mass, edesc, cons, groups, logs):
+        from . import _lib
+        torch, dev, n, N = self.torch, self.dev, self.n, self.N
+        f64, i32 = torch.float64, torch.int32
+        X, U, R, V, E, ST, ND, FA = logs
+        g = _lib.AdmmStep()
+        g.n, g.N, g.S, g.nroles, g.rho = n, N, S, len(groups), self.rho
+        g.leader_per_scenario, g.leader_len, g.T = int(lx.ndim == 3), lx.shape[-1], T
+        order = list(groups)
+        for i in range(n):
+            g.role_of[i] = order.index(self.role_of[i])
+        for r, fl in enumerate(order):
+            b = groups[fl]
+            b["params"] = torch.zeros((b["B"], b["cm"].n_param), dtype=f64, device=dev)
+            b["x0"] = torch.zeros((b["B"], 1, 2), dtype=f64, device=dev)
+            G = g.role[r]
+            for k, key in (("params", "params"), ("x0", "x0"), ("u", "u"), ("x", "x"), ("extra", "e"), ("modes", "mo"),
+                           ("status", "st"), ("nodes", "no")):
+                setattr(G, k, b[key].data_ptr())
+            G.has_front, G.has_back = int(not fl & FRONT), int(not fl & TRAILER)
+        table = groups[order[0]]["cm"].mode_gear
+        g.n_modes = len(table)
+        for k, gear in enumerate(table.tolist()):
+            g.mode_gear[k] = gear
+        t_idx = torch.zeros(1, dtype=torch.int64, device=dev)
+        r_idx = torch.zeros(1, dtype=i32, device=dev)
+        u0 = torch.empty((S, n), dtype=f64, device=dev)
+        gear0 = torch.empty((S, n), dtype=i32, device=dev) if self.friction else None
+        lead_t = torch.empty((S, 2), dtype=f64, device=dev)
+        x_cur = x.clone(); x_next = torch.empty_like(x_cur)
+        r_t = torch.empty(S, dtype=f64, device=dev); v_t = torch.empty(S, dtype=torch.uint8, device=dev)
+        e_t = torch.empty(S, dtype=i32, device=dev)
+        g.t, g.r, g.x, g.leader_x = t_idx.data_ptr(), r_idx.data_ptr(), x_cur.data_ptr(), lx.data_ptr()
+        for k, t_ in cons.items():
+            setattr(g, k, t_.data_ptr())
+        g.ND, g.failed_at, g.u0, g.U_log, g.ST = ND.data_ptr(), FA.data_ptr(), u0.data_ptr(), U.data_ptr(), ST.data_ptr()
+        g.gear0 = None if gear0 is None else gear0.data_ptr()
+
+        def piece(b):
+            return lambda: self._solve(b, b["x0"], b["params"])
+        pieces = [piece(b) for b in groups.values()]
         # Measured (r02, 1024 scenarios, n = 15, N = 8, 20 rounds x 3 timesteps): eager 1584 ms, round as a graph 1187 ms,
         # roles on forked streams 976 ms, both 1425 ms -- the MIQP rounds are kernel-bound (2.8 ms per interior launch), what
         # pays is running the two one-vehicle roles beside the interior one; inside a graph the branches did not overlap.
         fork = _Fork(torch, len(pieces), enabled=self.fork)
 
         def one_round():
-            # ---- x-update: all vehicles of a role in one launch, the roles side by side on forked streams ----
             fork.run(pieces)
-            if ar is not None:       # z / y update + next round's parameters: one kernel
-                api.admm_round_device(ar, ctx=self.ctx, stream=torch.cuda.current_stream().cuda_stream)
-                return
-            # ---- z-update: average of a vehicle's own prediction and its neighbours' copies of it (:421-447) ----
-            z[:, 0] = (xs[:, 0] + cf[:, 1]) / 2.0
-            z[:, n - 1] = (xs[:, n - 1] + cb[:, n - 2]) / 2.0
-            if n > 2:     # a TRUE division, as numpy's in the reference (torch turns `/ 3.0` into a product with 1/3: one ulp off)
-                z[:, 1:n - 1] = torch.div(xs[:, 1:n - 1] + cf[:, 2:] + cb[:, :n - 2], three)
-            # ---- y-update and the z each copy is pulled towards in the next round (:426-468) ----
-            y_front[:, 1:] += rho * (cf[:, 1:] - z[:, :-1])
-            y_back[:, :-1] += rho * (cb[:, :-1] - z[:, 1:])
-            zf[:, 1:] = z[:, :-1]
-            zb[:, :-1] = z[:, 1:]
+            api.admm_step_device(g, phase=_lib.ADMM_ROUND, ctx=self.ctx, stream=torch.cuda.current_stream().cuda_stream)
+            r_idx.add_(1)
 
-        # one consensus round = one CUDA graph (3 compiled-MPC solves + the z / y updates): the round, not the timestep,
-        # is the unit -- it repeats admm_iters times per timestep with nothing changing but the tensors it updates
+        # one consensus round = one CUDA graph (the role solves + the z / y update): the round, not the timestep, is the
+        # unit -- it repeats admm_iters times per timestep with nothing changing but the tensors it updates
         rnd = _StepGraph(torch, one_round, enabled=self.graph)
         stream = torch.cuda.current_stream().cuda_stream
-        for t in range(ep_len):
-            # coupling guesses from the previous step's predictions, shifted (fleet_naive_admm.py:392-402)
-            if have_pred:
+        for _ in range(T):
+            r_idx.zero_()
+            api.admm_step_device(g, phase=_lib.ADMM_PACK, ctx=self.ctx, stream=stream)
+            for _ in range(self.iters):
+                rnd()
+            api.admm_step_device(g, phase=_lib.ADMM_ADOPT, ctx=self.ctx, stream=stream)
+            lead_t.copy_(lx.index_select(-1, t_idx).squeeze(-1))                             # leader_x[:, t]
+            api.rollout_step_device(edesc, S, x_cur, u0, gear0, d_mass, lead_t, x_next, r_t, v_t, e_t, ctx=self.ctx,
+                                    stream=stream)
+            X.index_copy_(0, t_idx + 1, x_next.unsqueeze(0))
+            R.index_copy_(0, t_idx, r_t.unsqueeze(0))
+            V.index_copy_(0, t_idx, v_t.unsqueeze(0)); E.index_copy_(0, t_idx, e_t.unsqueeze(0))
+            x_cur.copy_(x_next)
+            t_idx.add_(1)
+        torch.cuda.synchronize()
+        rnd.close()
+
+    def _run_torch(self, S, T, x, lx, d_mass, edesc, cons, groups, logs):
+        torch, dev, n, N, rho = self.torch, self.dev, self.n, self.N, self.rho
+        f64, i32, np1 = torch.float64, torch.int32, N + 1
+        X, U, R, V, E, ST, ND, FA = logs
+        y_front, y_back, zf, zb, xs = (cons[k] for k in ("y_front", "y_back", "zf", "zb", "xs"))
+        if lx.ndim == 2:
+            lx = lx.unsqueeze(0).expand(S, -1, -1)
+        z = torch.zeros((S, n, 2, np1), dtype=f64, device=dev)
+        cf, cb = torch.zeros_like(z), torch.zeros_like(z)        # copies x_front / x_back of the last round
+        u0 = torch.empty((S, n), dtype=f64, device=dev)
+        stat = torch.empty((S, n), dtype=i32, device=dev)
+        nd = torch.empty((S, n), dtype=i32, device=dev)
+        x_cur = x.clone()                                         # state the rounds of this timestep start from
+        lwin = torch.empty((S, 1, 2 * np1), dtype=f64, device=dev)
+        three = torch.full((), 3.0, dtype=f64, device=dev)
+        zero = torch.zeros((), dtype=f64, device=dev)
+        ar = torch.arange(n, device=dev)
+
+        def role_piece(fl, g):
+            def piece():
+                idx, k, B = g["idx"], g["k"], g["B"]
+                params = torch.cat((lwin.expand(S, k, -1), y_front[:, idx].reshape(S, k, -1), zf[:, idx].reshape(S, k, -1),
+                                    y_back[:, idx].reshape(S, k, -1), zb[:, idx].reshape(S, k, -1)), dim=2).reshape(B, -1).contiguous()
+                x0g = x_cur.view(S, n, 2)[:, idx].reshape(B, 1, 2).contiguous()
+                self._solve(g, x0g, params)
+                # a solve that is not optimal contributes zeros (solve_mpc(raises=False), LocalMpcADMM._post)
+                st = g["st"].view(S, k)
+                ok = (st == 2).view(S, k, 1, 1)
+                xs[:, idx] = torch.where(ok, g["x"].view(S, k, 2, np1), zero)
+                u0[:, idx] = torch.where(ok[:, :, 0, 0], g["u"].view(S, k, N)[:, :, 0], zero)
+                stat[:, idx] = st
+                nd[:, idx] = g["no"].view(S, k)
+                e = g["e"].view(S, k, -1)
+                o = 0
+                if not fl & FRONT:
+                    cf[:, idx] = torch.where(ok, e[:, :, o:o + 2 * np1].reshape(S, k, 2, np1), zero); o += 2 * np1
+                if not fl & TRAILER:
+                    cb[:, idx] = torch.where(ok, e[:, :, o:o + 2 * np1].reshape(S, k, 2, np1), zero)
+            return piece
+        pieces = [role_piece(fl, g) for fl, g in groups.items()]
+        fork = _Fork(torch, len(pieces), enabled=self.fork)
+        stream = torch.cuda.current_stream().cuda_stream
+        for t in range(T):
+            if t > 0:       # coupling guesses from the previous step's predictions, shifted (fleet_naive_admm.py:392-402)
                 sh = torch.cat((xs[..., 1:], xs[..., -1:]), dim=-1)
                 zf[:, 1:] = sh[:, :-1]
                 zb[:, :-1] = sh[:, 1:]
             lwin.copy_(lx[:, :, t:t + np1].reshape(S, 1, 2 * np1))
             x_cur.copy_(x)
-            if ar is not None:       # this timestep's states and first parameter vectors of every role
-                for g in groups.values():
-                    g["x0"].copy_(x_cur.view(S, n, 2)[:, g["idx"]].reshape(g["B"], 1, 2))
-                api.admm_round_device(ar, pack_only=True, ctx=self.ctx, stream=stream)
-            for _ in range(self.iters):
-                rnd()
-            if ar is not None:       # inputs and statuses of the last round
-                for g in groups.values():
-                    u0[:, g["idx"]] = g["u"].view(S, g["k"], N)[:, :, 0]
-                    stat[:, g["idx"]] = g["st"].view(S, g["k"])
-            have_pred = True
+            for r in range(self.iters):
+                # ---- x-update: all vehicles of a role in one launch, the roles side by side on forked streams ----
+                fork.run(pieces)
+                # ---- z-update: average of a vehicle's own prediction and its neighbours' copies of it (:421-447) ----
+                z[:, 0] = (xs[:, 0] + cf[:, 1]) / 2.0
+                z[:, n - 1] = (xs[:, n - 1] + cb[:, n - 2]) / 2.0
+                if n > 2:     # a TRUE division, as numpy's in the reference (torch turns `/ 3.0` into a product with 1/3: one ulp off)
+                    z[:, 1:n - 1] = torch.div(xs[:, 1:n - 1] + cf[:, 2:] + cb[:, :n - 2], three)
+                # ---- y-update and the z each copy is pulled towards in the next round (:426-468) ----
+                y_front[:, 1:] += rho * (cf[:, 1:] - z[:, :-1])
+                y_back[:, :-1] += rho * (cb[:, :-1] - z[:, 1:])
+                zf[:, 1:] = z[:, :-1]
+                zb[:, :-1] = z[:, 1:]
+                # ---- logs: largest node count, first solve that was not optimal (lowest vehicle index) ----
+                ND[t] = torch.maximum(ND[t], nd.max(dim=1).values)
+                bad = stat != 2
+                first = torch.where(bad, ar, n).min(dim=1).values
+                new = (FA[:, 0] < 0) & (first < n)
+                row = torch.stack((torch.full_like(first, t), torch.full_like(first, r),
+                                   stat.gather(1, first.clamp(max=n - 1).unsqueeze(1)).squeeze(1)), dim=1).to(i32)
+                FA.copy_(torch.where(new.unsqueeze(1), row, FA))
             U[t] = u0
             ST[t] = stat
             api.rollout_step_device(edesc, S, x, U[t], None, d_mass, lx[:, :, t].contiguous(), X[t + 1], R[t], V[t],
                                     E[t], ctx=self.ctx, stream=stream)
             x = X[t + 1]
-        torch.cuda.synchronize()
-        rnd.close()
-        return dict(X=X.cpu().numpy(), U=U.cpu().numpy(), R=R.cpu().numpy(), violations=V.cpu().numpy(),
-                    errors=E.cpu().numpy(), status=ST.cpu().numpy())
 
 
 class BatchedSeqSweep(BatchedDecentSweep):

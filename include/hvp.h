@@ -309,6 +309,61 @@ typedef struct {
 } hvp_admm_round;
 int hvp_admm_round_dev(hvp_ctx* ctx, const hvp_admm_round* g, void* stream);
 
+/* ---- fused glue of a naive-ADMM timestep ----------------------------------------------------------------------
+ * What ADMMCoordinator.get_control / on_timestep_end (fleet_naive_admm.py:379-587) do around the role solves, for all
+ * S scenarios at once, one thread per (scenario, vehicle); the z / y update is the device code of hvp_admm_round_dev.
+ * role_of[i] = index into role[] of vehicle i; the problems of a role (the rows of its hvp_mpc_solve_dev call) are
+ * ordered [scenario][vehicle of the role].  t and the round index r are read from DEVICE memory (the caller advances
+ * them) so that a round can be replayed as a CUDA graph.  A vehicle whose solve is not optimal (status != 2)
+ * contributes zeros for its own prediction and its copies and gets u0 = 0 and gear 6, as solve_mpc(raises=False)
+ * gives it (LocalMpcADMM._post).  Three phases:
+ *   HVP_ADMM_PACK  (start of a timestep, before round 0): the role rows x0 = x[s][i]; when t > 0 the shifted previous
+ *       predictions zf[i] = xs[i-1], zb[i] = xs[i+1] with column 0 dropped and the last one repeated (no re-extrapolated
+ *       position: get_predicted_state(shifted=True)); then the parameter rows [lwin | y_front | zf | y_back | zb],
+ *       lwin = leader_x[:, t : t+N+1] (a column past the end of leader_x reads its last column).
+ *   HVP_ADMM_ROUND (after the role solves of round r): xs, zf, zb, y_front, y_back and the parameter rows exactly as
+ *       hvp_admm_round_dev (same order of additions, a true division by 3), lwin as in PACK;
+ *       ND[t][s] = max(ND[t][s], nodes of every vehicle); failed_at[s] = (t, r, status) of the first solve of the
+ *       episode that was not optimal -- the lowest vehicle index within the first such round -- (-1, -1, 0): none;
+ *       the row is reset at t == 0, r == 0.
+ *   HVP_ADMM_ADOPT (after the last round, before the rollout): u0 = u[..., 0], with a gear output gear0 =
+ *       mode_gear[modes[..., 0]] (mode index clamped to [0, n_modes)); U_log[t] = u0, followed by the gears as doubles
+ *       when gear0 is given (w = 2n: the reference's [u_g ; gears]; else w = n); ST[t] = the last round's statuses.
+ * ND, failed_at, U_log and ST are written only for 0 <= t < T.  All pointers are device pointers. */
+#define HVP_ADMM_PACK 0
+#define HVP_ADMM_ROUND 1
+#define HVP_ADMM_ADOPT 2
+typedef struct {
+    double* params;               /* PACK / ROUND out: [rows][5 * 2(N+1)] */
+    double* x0;                   /* PACK out: [rows][1][2] */
+    const double* u; const double* x; const double* extra; const int32_t* modes; const int32_t* status;
+    const int32_t* nodes;         /* solve outputs: [rows][N], [rows][2][N+1], [rows][ne], [rows][N], [rows], [rows] */
+    int32_t has_front, has_back;  /* the role's formulation holds an x_front / x_back copy (not FRONT / not TRAILER) */
+} hvp_admm_step_role;
+typedef struct {
+    int32_t n, N, S, phase;       /* phase: HVP_ADMM_PACK | HVP_ADMM_ROUND | HVP_ADMM_ADOPT */
+    int32_t nroles;               /* 1..4 */
+    int32_t leader_per_scenario;  /* leader_x is [S][2][leader_len] (1) or [2][leader_len] shared (0) */
+    int64_t leader_len;           /* PACK / ROUND: columns of the leader trajectory (>= 1) */
+    int64_t T;                    /* ROUND / ADOPT: rows of the episode logs */
+    double rho;
+    int32_t n_modes;              /* ADOPT with gear0: entries of mode_gear (1..16) */
+    int32_t reserved;
+    int32_t mode_gear[16];
+    hvp_admm_step_role role[4];
+    int32_t role_of[64];
+    const int64_t* t;             /* device pointer: timestep index */
+    const int32_t* r;             /* device pointer: round index within the timestep (ROUND) */
+    const double* x;              /* PACK: [S][n][2] */
+    const double* leader_x;       /* PACK / ROUND */
+    double* y_front; double* y_back; double* zf; double* zb; double* xs; /* [S][n][2][N+1] each */
+    int32_t* ND;                  /* ROUND: [T][S] */
+    int32_t* failed_at;           /* ROUND: [S][3] */
+    double* u0; int32_t* gear0;   /* ADOPT out: [S][n] each; gear0 NULL: no gears */
+    double* U_log; int32_t* ST;   /* ADOPT: [T][S][w], [T][S][n] */
+} hvp_admm_step;
+int hvp_admm_step_dev(hvp_ctx* ctx, const hvp_admm_step* g, void* stream);
+
 /* ---- fused glue of a centralized timestep ---------------------------------------------------------------------
  * What TrackingCentralizedAgent (fleet_cent_mld.py:22-32) and MpcMldCent / MpcGearCent.solve_mpc (mpcs/mpc_gear.py:
  * 116-135) do around the solve, for all S scenarios at once, one thread per (scenario, vehicle).  t is read from DEVICE
