@@ -137,10 +137,10 @@ struct FlatSolver {
     bool slab_ok;                                       // ... and nothing has been built since (warm start of its first child)
     // active set
     int q;
-    uint64_t act_lo, act_hi;                            // slot ids, 8 bits each
+    uint64_t act_lo, act_hi;                            // slot bytes (act_raw), 8 bits each
     uint32_t satf, satb;
     // constraint being added
-    int pid, pkind, pj;
+    int pcode, pkind, pj;                               // pcode: p's slot byte once it is added (act_raw)
     double psgn, pcoef, nHn, lam_p, cp;
     double dual;                                         // value of the node's dual function (lower bound)
     bool p_soft;
@@ -154,6 +154,10 @@ struct FlatSolver {
 #endif
     }
     HVP_HD static int tri(int a, int b) { return a * (a + 1) / 2 + b; }          // a >= b
+    // max / min of operands that are never NaN (parameters, merged bounds): a compare and two selects instead of the
+    // NaN handling of fmax / fmin
+    HVP_HD static double nmax(double a, double b) { return a > b ? a : b; }
+    HVP_HD static double nmin(double a, double b) { return a < b ? a : b; }
     HVP_HD double ra(int rg) const { return rg < 4 ? a_lo : a_hi; }
     HVP_HD double rc(int rg) const { return rg < 4 ? c_lo : c_hi; }
     HVP_HD double rb(int rg) const { return P->bgear[rg] * inv_m; }
@@ -162,17 +166,34 @@ struct FlatSolver {
     HVP_HD void set_mode(int k, int rg) { modes_pk = (modes_pk & ~(7ull << (3 * k))) | ((uint64_t)rg << (3 * k)); }
     HVP_HD int cand(int lv) const { return (int)((cand_pk >> (7 * lv)) & 0x7fu); }
     HVP_HD void set_cand(int lv, int v) { cand_pk = (cand_pk & ~(0x7full << (7 * lv))) | ((uint64_t)v << (7 * lv)); }
-    // slot a's row: id = type * 12 + stage in the low 7 bits, bit 7 = the row enters with sign -1 (the sign
-    // includes a soft row's orientation at the time it became active; it cannot flip while active)
-    HVP_HD int act_raw(int a) const { return (int)(((a < 8 ? act_lo >> (8 * a) : act_hi >> (8 * (a - 8)))) & 0xffu); }
-    HVP_HD int act(int a) const { return act_raw(a) & 0x7f; }
-    HVP_HD double slot_sgn(int a) const { return (act_raw(a) & 0x80) ? -1.0 : 1.0; }
-    HVP_HD double slot_coef(int a) const {           // difference coefficient: a_r of the stage for input-limit rows
-        const int id = act(a), t = id / 12;
-        return (t == T_UHI || t == T_ULO) ? ra(mode(id - 12 * t)) : 1.0;
+    // Slot a's row is one byte, decoded when the row enters the active set so that the products over the active set
+    // read it with masks only: bits 0-3 = stage j, bit 4 = the row enters with sign -1 (the sign includes a soft row's
+    // orientation at the time it became active; it cannot flip while active), bits 5-7 = row class (R_*), which fixes
+    // the row's shape and, for input-limit rows, its difference coefficient a_r (the region of stage j is fixed for the
+    // whole node).  A (class, sign, stage) byte identifies the row: UB / LB, ACC / DEC, ... differ in the sign bit.
+    enum : int { R_BOUND = 0, R_ACC, R_IN_LO, R_IN_HI, R_POS, R_SF, R_SB };
+    // row class of each constraint type (miqp_core.cuh T_*), 4 bits per type; input-limit rows add 1 in regions >= 4
+    static constexpr uint64_t kClassOfType = 0x6544221100ull;
+    // q <= N (a row dependent on the active set is never added), so act_hi is only used at N = 9
+    HVP_HD int act_raw(int a) const { return (int)((((N <= 8 || a < 8) ? act_lo >> (8 * a) : act_hi >> (8 * (a - 8)))) & 0xffu); }
+    HVP_HD static bool slot_soft(int b) { return b >= (R_SF << 5); }
+    HVP_HD double slot_coef(int b) const {           // difference coefficient: a_r of the stage for input-limit rows
+        const int cls = b >> 5;
+        return cls == R_IN_LO ? a_lo : (cls == R_IN_HI ? a_hi : 1.0);
     }
+    // the slot bytes in order, from a copy of act_lo / act_hi shifted by one slot per call (constant shifts)
+    struct SlotIter {
+        uint64_t lo, hi;
+        HVP_HD int next() {
+            const int b = (int)(lo & 0xffu);
+            lo >>= 8;
+            if (N > 8) { lo |= hi << 56; hi >>= 8; }
+            return b;
+        }
+    };
+    HVP_HD SlotIter slots() const { return SlotIter{act_lo, act_hi}; }
     HVP_HD void set_act(int a, int id) {
-        if (a < 8) act_lo = (act_lo & ~(0xffull << (8 * a))) | ((uint64_t)id << (8 * a));
+        if (N <= 8 || a < 8) act_lo = (act_lo & ~(0xffull << (8 * a))) | ((uint64_t)id << (8 * a));
         else act_hi = (act_hi & ~(0xffull << (8 * (a - 8)))) | ((uint64_t)id << (8 * (a - 8)));
     }
     HVP_HD double Hoff(int j) const { return hw1 * (double)(N - 1 - j) + hw2; }
@@ -379,8 +400,9 @@ struct FlatSolver {
         HVP_ROLL
         for (int i = 0; i < N; ++i) w(LY::O_YP, i) = w(LY::O_HINV, pj0 * N + i);
         const double nHn0 = w(LY::O_HINV, pj0 * N + pj0);
+        SlotIter si = slots();
         HVP_ROLL
-        for (int a = 0; a < q; ++a) w(LY::O_D, a) = slot_dot(a, LY::O_YP);
+        for (int a = 0; a < q; ++a) w(LY::O_D, a) = slot_dot(si.next(), LY::O_YP);
         double nz = nHn0, tp = INF, tm = INF;
         HVP_ROLL
         for (int a = 0; a < q; ++a) {
@@ -393,7 +415,7 @@ struct FlatSolver {
             for (int b = a + 1; b < q; ++b) { s += w(LY::O_GINV, gi) * w(LY::O_D, b); gi += b + 1; }
             nz -= s * w(LY::O_D, a);
             const double la = w(LY::O_LAM, a);
-            const bool soft = act(a) >= T_SF * 12;
+            const bool soft = slot_soft(act_raw(a));
             if (s > 1e-14) {
                 const double is = hvp_rcp(s);
                 tp = fmin(tp, la * is);
@@ -570,8 +592,9 @@ struct FlatSolver {
         slab_ok = false;
         if (warm) {
             const double den = rank1(L - 1, mode(L - 1), 1.0);              // v = H^-1 e in O_WV
+            SlotIter si = slots();
             HVP_ROLL
-            for (int a = 0; a < q; ++a) w(LY::O_R, a) = slot_dot(a, LY::O_WV);   // z = N'v
+            for (int a = 0; a < q; ++a) w(LY::O_R, a) = slot_dot(si.next(), LY::O_WV);   // z = N'v
             double zr = 0.0;
             HVP_ROLL
             for (int a = 0; a < q; ++a) {                                    // r = Ginv z  (into O_YP)
@@ -632,16 +655,17 @@ struct FlatSolver {
         if (warm) {
             // residual c_a = n_a'x_u - rhs_a of the parent's rows: a bound row's right-hand side may have moved
             // (the region of the newly fixed stage), every other row was active at x*: c_a = n_a'(x_u - x*)
+            SlotIter si = slots();
             HVP_ROLL
             for (int a = 0; a < q; ++a) {
-                const int id = act(a), t = id / 12, j = id - 12 * t;
+                const int b = si.next(), j = b & 15;
                 double cv;
-                if (t <= T_LB) {
+                if ((b >> 5) == R_BOUND) {
                     double lo, hi;
                     bounds(j, lo, hi);
-                    cv = (t == T_UB) ? w(LY::O_X, j) - hi : lo - w(LY::O_X, j);
+                    cv = (b & 16) ? lo - w(LY::O_X, j) : w(LY::O_X, j) - hi;     // LB : UB
                 } else {
-                    cv = slot_dot(a, LY::O_R);
+                    cv = slot_dot(b, LY::O_R);
                 }
                 w(LY::O_YP, a) = cv;
             }
@@ -658,7 +682,7 @@ struct FlatSolver {
                 for (int b = a + 1; b < q; ++b) { s += w(LY::O_GINV, gi) * w(LY::O_YP, b); gi += b + 1; }
                 w(LY::O_LAM, a) = s;
                 cl += s * w(LY::O_YP, a);
-                if (!(s >= 0.0) || (act(a) >= T_SF * 12 && s > ww)) ok = false;
+                if (!(s >= 0.0) || (slot_soft(act_raw(a)) && s > ww)) ok = false;
             }
 #ifdef HVP_DEBUG_STATS
             if (ok) g_warm[2] += 1; was_warm = ok;
@@ -667,8 +691,9 @@ struct FlatSolver {
                 // x = x_u - H^-1 N lambda ; dual value = f(x_u) + c'lambda / 2
                 HVP_ROLL
                 for (int i = 0; i < N; ++i) w(LY::O_WV, i) = 0.0;
+                SlotIter sj = slots();
                 HVP_ROLL
-                for (int a = 0; a < q; ++a) slot_axpy(a, w(LY::O_LAM, a), LY::O_WV);
+                for (int a = 0; a < q; ++a) slot_axpy(sj.next(), w(LY::O_LAM, a), LY::O_WV);
                 double wr[N];
                 HVP_FLAT_UNROLL
                 for (int j = 0; j < N; ++j) wr[j] = w(LY::O_WV, j);
@@ -694,13 +719,13 @@ struct FlatSolver {
         if (kHull && j >= L) { lo = fmax(lo, C->rlo[j + 1]); hi = fmin(hi, C->rhi[j + 1]); }
         if (j + 1 < L) {
             const int rg = mode(j + 1);
-            lo = fmax(lo, P->edge[rg]); hi = fmin(hi, P->edge[rg + 1]);
+            lo = nmax(lo, P->edge[rg]); hi = nmin(hi, P->edge[rg + 1]);
         }
         if (j == 0) {
             const int r0 = mode(0);
             const double m = ra(r0) * v0 + rc(r0), bb = rb(r0);
-            lo = fmax(lo, fmax(v0 + P->a_dec, m + bb * P->umin));
-            hi = fmin(hi, fmin(v0 + P->a_acc, m + bb * P->umax));
+            lo = nmax(lo, nmax(v0 + P->a_dec, m + bb * P->umin));
+            hi = nmin(hi, nmin(v0 + P->a_acc, m + bb * P->umax));
         }
     }
 
@@ -719,7 +744,7 @@ struct FlatSolver {
 #define HVP_CAND(T, J, S)                                              \
     {                                                                  \
         const double s__ = (S);                                        \
-        if (s__ > lb) { lb = s__; li = (T) * 12 + (J); }               \
+        if (s__ > lb) { lb = s__; li = (T) * 16 + (J); }               \
     }
         HVP_FLAT_UNROLL
         for (int j = 0; j < N; ++j) {
@@ -760,11 +785,24 @@ struct FlatSolver {
             if (bj[j] > best) { best = bj[j]; bid = ij[j]; }
 #undef HVP_CAND
         if (bid >= 0) {
+            // p = row (type pt, stage pj) and the slot byte it will have (act_raw)
+            const int pt = bid >> 4;
+            pj = bid & 15;
+            int cls = (int)((kClassOfType >> (4 * pt)) & 7u);
+            if (cls == R_IN_LO && mode(pj) >= 4) cls = R_IN_HI;
+            pkind = cls == R_BOUND ? 0 : (cls < R_POS ? 1 : 2);
+            psgn = (pt & 1) ? -1.0 : 1.0;
+            if (pt == T_SF) psgn = ((satf >> pj) & 1u) ? -1.0 : 1.0;
+            if (pt == T_SB) psgn = ((satb >> pj) & 1u) ? 1.0 : -1.0;
+            pcode = pj | (psgn < 0.0 ? 16 : 0) | (cls << 5);
+            pcoef = slot_coef(pcode);
+            p_soft = cls >= R_SF;
             // The most violated row is already active: its residual is round-off drift (ill-conditioned,
             // heavily constrained node) and every other row is violated by even less -> converged.
             bool dup = false;
+            SlotIter si = slots();
             HVP_ROLL
-            for (int a = 0; a < q; ++a) dup = dup || (act(a) == bid);
+            for (int a = 0; a < q; ++a) dup = dup || (si.next() == pcode);
             if (dup) {
                 if (best < 1e-6) bid = -1;
                 else { node_done(2, 0.0); return; }
@@ -792,15 +830,6 @@ struct FlatSolver {
             node_done(0, f);
             return;
         }
-        pid = bid;
-        const int pt = pid / 12;
-        pj = pid - 12 * pt;
-        pkind = (pt < T_ACC) ? 0 : (pt < T_PHI ? 1 : 2);
-        psgn = (pt & 1) ? -1.0 : 1.0;
-        pcoef = (pt == T_UHI || pt == T_ULO) ? ra(mode(pj)) : 1.0;
-        if (pt == T_SF) psgn = ((satf >> pj) & 1u) ? -1.0 : 1.0;
-        if (pt == T_SB) psgn = ((satb >> pj) & 1u) ? 1.0 : -1.0;
-        p_soft = pt >= T_SF;
         // yp = H^-1 n_p and nHn = n_p' yp
         double acc = 0.0;
         HVP_ROLL
@@ -826,24 +855,24 @@ struct FlatSolver {
         state = S_STEP;
     }
 
-    // n_a' v for slot a's row, v in the work array at `off`
-    HVP_HD double slot_dot(int a, int off) const {
-        const int id = act(a), t = id / 12, j = id - 12 * t;
+    // n' v for the row of slot byte b, v in the work array at `off`
+    HVP_HD double slot_dot(int b, int off) const {
+        const int j = b & 15, cls = b >> 5;
         double s;
-        if (t < T_ACC) s = w(off, j);
-        else if (t < T_PHI) s = w(off, j) - slot_coef(a) * w(off, j - 1);
+        if (cls == R_BOUND) s = w(off, j);
+        else if (cls < R_POS) s = w(off, j) - slot_coef(b) * w(off, j - 1);
         else {
             s = 0.0;
             HVP_ROLL
             for (int i = 0; i < j; ++i) s += w(off, i);
         }
-        return slot_sgn(a) * s;
+        return (b & 16) ? -s : s;
     }
-    HVP_HD void slot_axpy(int a, double c0, int off) const {
-        const int id = act(a), t = id / 12, j = id - 12 * t;
-        const double c = c0 * slot_sgn(a);
-        if (t < T_ACC) w(off, j) += c;
-        else if (t < T_PHI) { w(off, j) += c; w(off, j - 1) -= c * slot_coef(a); }
+    HVP_HD void slot_axpy(int b, double c0, int off) const {
+        const int j = b & 15, cls = b >> 5;
+        const double c = (b & 16) ? -c0 : c0;
+        if (cls == R_BOUND) w(off, j) += c;
+        else if (cls < R_POS) { w(off, j) += c; w(off, j - 1) -= c * slot_coef(b); }
         else {
             HVP_ROLL
             for (int i = 0; i < j; ++i) w(off, i) += c;
@@ -860,8 +889,9 @@ struct FlatSolver {
         const bool zero_step = (cp <= tol);
         if (zero_step && !(lam_p > 0.0)) { state = S_SELECT; return; }
         // d = N' yp ; r = Ginv d ; nz = nHn - d'r
+        SlotIter si = slots();
         HVP_ROLL
-        for (int a = 0; a < q; ++a) w(LY::O_D, a) = slot_dot(a, LY::O_YP);
+        for (int a = 0; a < q; ++a) w(LY::O_D, a) = slot_dot(si.next(), LY::O_YP);
         double nz = nHn;
         // ratio tests without a division per slot: keep the best (numerator, denominator) pair
         double n1 = 1.0, d1 = 0.0, n3 = 1.0, d3 = 0.0;
@@ -880,7 +910,7 @@ struct FlatSolver {
             const double la = w(LY::O_LAM, a);
             if (s > 1e-14) {
                 if (k1 < 0 || la * d1 < n1 * s) { n1 = la; d1 = s; k1 = a; }
-            } else if (s < -1e-14 && act(a) >= T_SF * 12) {
+            } else if (s < -1e-14 && slot_soft(act_raw(a))) {
                 const double num = ww - la, den = -s;
                 if (k3 < 0 || num * d3 < n3 * den) { n3 = num; d3 = den; k3 = a; }
             }
@@ -908,8 +938,9 @@ struct FlatSolver {
                 else v = (i < pj) ? psgn : 0.0;
                 w(LY::O_WV, i) = v;
             }
+            SlotIter sj = slots();
             HVP_ROLL
-            for (int a = 0; a < q; ++a) slot_axpy(a, -w(LY::O_R, a), LY::O_WV);
+            for (int a = 0; a < q; ++a) slot_axpy(sj.next(), -w(LY::O_R, a), LY::O_WV);
             double wr[N];
             HVP_FLAT_UNROLL
             for (int j = 0; j < N; ++j) wr[j] = w(LY::O_WV, j);
@@ -936,14 +967,14 @@ struct FlatSolver {
                 w(LY::O_GINV, tri(q, a)) = -ra_;
             }
             w(LY::O_GINV, tri(q, q)) = is;
-            set_act(q, pid | (psgn < 0.0 ? 0x80 : 0));
+            set_act(q, pcode);
             w(LY::O_LAM, q) = lam_p;
             ++q;
             state = S_SELECT;
             return;
         }
         if (t == t3p) {                                          // soft p saturates: flip, not added
-            if (pid / 12 == T_SF) satf ^= (1u << pj); else satb ^= (1u << pj);
+            if ((pcode >> 5) == R_SF) satf ^= (1u << pj); else satb ^= (1u << pj);
             state = S_SELECT;
             return;
         }
@@ -951,8 +982,8 @@ struct FlatSolver {
         if (t == t1) drop = k1;
         else {                                                   // active soft row saturates: flip + drop
             drop = k3;
-            const int id = act(drop), j = id % 12;
-            if (id / 12 == T_SF) satf ^= (1u << j); else satb ^= (1u << j);
+            const int b = act_raw(drop), j = b & 15;
+            if ((b >> 5) == R_SF) satf ^= (1u << j); else satb ^= (1u << j);
         }
         {   // Ginv <- Ginv - g_k g_k'/g_kk, then delete row/column `drop` (packed, in place)
             const double ikk = hvp_rcp(w(LY::O_GINV, tri(drop, drop)));
