@@ -83,6 +83,9 @@ struct CoopSolver {
         hw1 = 2.0 * wp * nterm;
         hw2 = 2.0 * wp * (tf ? t0 : 0.0);
         hd = 2.0 * wp * (tf ? t0 * t0 : 0.0) + 2.0 * wvv * nterm;
+        // no reference term (a front vehicle that is also the trailer and not the leader): the Hessian is the input
+        // cost of the fixed stages alone, singular at every node that leaves a stage free -- only leaves are solved
+        notrack = nterm < 0.5;
         const I ln = bk.lane();
         const Bm valid = ln < N;
         const I kk = ln + 1;                       // lane j holds stage k = j+1
@@ -142,6 +145,7 @@ struct CoopSolver {
     double inc, nlo_cur, nhi_cur;
     double dual;                 // value of the node's dual function: lower bound on the node optimum
     bool dive;                   // first descent: path nodes are not solved, only the leaf
+    bool notrack;                // no reference term: no node but a leaf is solved (setup)
     uint64_t best_modes, cand_lo, cand_hi;
     bool trouble, limit, timeout;
     long long t_start;
@@ -223,11 +227,11 @@ struct CoopSolver {
             rlo = bk.sel(ln == lev, bk.splat(nlo - eps), rlo);
             rhi = bk.sel(ln == lev, bk.splat(nhi + eps), rhi);
             L = lev + 1;
-            if (dive && nodes >= 1 && L < N) {
+            if (((dive && nodes >= 1) || notrack) && L < N) {
                 // first descent (see flat_core.cuh): without an incumbent the relaxations along the path
                 // cannot prune; follow the last relaxed trajectory and solve the leaf directly
                 ++lev;
-                xstar = bk.sel(ln == lev, bk.splat(bk.bcast(x, lev - 1)), xstar);
+                xstar = bk.sel(ln == lev, bk.splat(notrack ? bk.bcast(xstar, lev - 1) : bk.bcast(x, lev - 1)), xstar);
                 int cn = 0;
                 for (int c = 0; c < NREG; ++c)
                     if (P->edge[c] <= nhi_cur + eps && P->edge[c + 1] >= nlo_cur - eps) cn |= (1 << c);

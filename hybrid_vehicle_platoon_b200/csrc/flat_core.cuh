@@ -127,6 +127,7 @@ struct FlatSolver {
     uint64_t modes_pk, best_modes, cand_pk, built_pk;   // 3 bits / stage; 7 candidate bits / level
     int built_L;                                        // H^-1 currently holds stages 0..built_L-1 of built_pk
     bool trouble, limit, timeout;
+    bool notrack;                                       // no reference term: only leaves are solved
     bool dive;                                          // first descent: path nodes are not solved, only the leaf
     bool hinted;                                        // the node being solved is the caller's hinted leaf
     int hint_c0;
@@ -259,33 +260,14 @@ struct FlatSolver {
         }
         sfv[0] = sbv[0] = 0.0;
         // ---- H^-1 of the pure tracking Hessian (no stage fixed): one of three matrices the host inverted ----
-        if (nterm > 0.5) {
+        // Without a reference term (a front vehicle that is also the trailer and not the leader) the Hessian is the
+        // input cost of the fixed stages alone: singular at every node that leaves a stage free.  Such a problem is
+        // searched over its leaves only (do_next), and each leaf inverts its own Hessian (leaf_inverse).
+        notrack = nterm < 0.5;
+        if (!notrack) {
             const double* h0 = P->h0inv[tf ? (tb ? 2 : 1) : 0];
             HVP_ROLL
             for (int e = 0; e < N * N; ++e) w(LY::O_HINV, e) = h0[e];
-        } else {
-            // no reference term at all (a front vehicle that is also the trailer and not the leader): the Hessian
-            // is singular until a stage is fixed; keep the in-place Gauss-Jordan for this degenerate case
-            HVP_ROLL
-            for (int i = 0; i < N; ++i) {
-                HVP_ROLL
-                for (int j = 0; j < N; ++j) w(LY::O_HINV, i * N + j) = (i == j) ? Hdiag(i) : Hoff(i > j ? i : j);
-            }
-            HVP_ROLL
-            for (int k = 0; k < N; ++k) {
-                const double pinv = hvp_rcp(w(LY::O_HINV, k * N + k));
-                HVP_ROLL
-                for (int j = 0; j < N; ++j) w(LY::O_HINV, k * N + j) *= pinv;
-                w(LY::O_HINV, k * N + k) = pinv;
-                HVP_ROLL
-                for (int i = 0; i < N; ++i) {
-                    if (i == k) continue;
-                    const double f = w(LY::O_HINV, i * N + k);
-                    HVP_ROLL
-                    for (int j = 0; j < N; ++j)
-                        w(LY::O_HINV, i * N + j) = (j == k) ? -f * pinv : w(LY::O_HINV, i * N + j) - f * w(LY::O_HINV, k * N + j);
-                }
-            }
         }
         built_L = 0; built_pk = 0;
         // ---- start of the search ----
@@ -469,12 +451,13 @@ struct FlatSolver {
             if (pc > P->pmax + eps || pc < P->pmin - eps) continue;
             C->rlo[lev + 1] = nlo - eps; C->rhi[lev + 1] = nhi + eps;
             L = lev + 1;
-            if (dive && nodes >= 1 && L < N) {
+            if (((dive && nodes >= 1) || notrack) && L < N) {
                 // First descent: no incumbent exists yet, so the relaxations along the path could not
                 // prune anything -- they only guide the choice of region.  Keep following the last
                 // relaxed trajectory and solve the LEAF directly; its objective is the first incumbent.
+                // (notrack: every descent, as the oracle enumerates the leaves; no relaxation is solved.)
                 ++lev;
-                C->xstar[lev] = w(LY::O_X, lev - 1);
+                C->xstar[lev] = notrack ? C->xstar[lev - 1] : w(LY::O_X, lev - 1);
                 if (ALG2) C->pf[lev] = -HUGE_VAL;        // no solved parent: no sibling bound at this level
                 int cn = 0;
                 HVP_ROLL
@@ -577,6 +560,42 @@ struct FlatSolver {
         return den;                                        // H'^-1 = H^-1 - den v v', v left in O_WV
     }
 
+    // H^-1 of a leaf of a problem without reference terms (notrack): H = sum over the stages of the input cost
+    // 2 qu e e', e = (e_k - a e_{k-1})/b, tridiagonal and positive definite once every stage is fixed;
+    // in-place Gauss-Jordan (no pivoting needed)
+    HVP_HD void leaf_inverse() {
+        const double qu2 = 2.0 * P->qu;
+        HVP_ROLL
+        for (int e = 0; e < N * N; ++e) w(LY::O_HINV, e) = 0.0;
+        HVP_ROLL
+        for (int k = 0; k < N; ++k) {
+            const int rg = mode(k);
+            const double ib = hvp_rcp(rb(rg));
+            w(LY::O_HINV, k * N + k) += qu2 * ib * ib;
+            if (k >= 1) {
+                const double ea = -ra(rg) * ib;
+                w(LY::O_HINV, (k - 1) * N + k - 1) += qu2 * ea * ea;
+                w(LY::O_HINV, k * N + k - 1) += qu2 * ea * ib;
+                w(LY::O_HINV, (k - 1) * N + k) += qu2 * ea * ib;
+            }
+        }
+        HVP_ROLL
+        for (int k = 0; k < N; ++k) {
+            const double pinv = hvp_rcp(w(LY::O_HINV, k * N + k));
+            HVP_ROLL
+            for (int j = 0; j < N; ++j) w(LY::O_HINV, k * N + j) *= pinv;
+            w(LY::O_HINV, k * N + k) = pinv;
+            HVP_ROLL
+            for (int i = 0; i < N; ++i) {
+                if (i == k) continue;
+                const double f = w(LY::O_HINV, i * N + k);
+                HVP_ROLL
+                for (int j = 0; j < N; ++j)
+                    w(LY::O_HINV, i * N + j) = (j == k) ? -f * pinv : w(LY::O_HINV, i * N + j) - f * w(LY::O_HINV, k * N + j);
+            }
+        }
+    }
+
     // ---- BUILD: bring H^-1 to this node, gradient, unconstrained minimiser -----------------
     HVP_HD void do_build() {
         const double qu = P->qu, ww = P->w;
@@ -615,6 +634,8 @@ struct FlatSolver {
                 HVP_ROLL
                 for (int b = 0; b <= a; ++b) w(LY::O_GINV, tri(a, b)) += ra_ * w(LY::O_YP, b);
             }
+        } else if (notrack) {
+            leaf_inverse();
         } else {
             HVP_ROLL
             for (int k = built_L - 1; k >= c; --k) rank1(k, mode_of(built_pk, k), -1.0);

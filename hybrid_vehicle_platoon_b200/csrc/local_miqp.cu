@@ -180,12 +180,15 @@ flat_miqp_kernel(const __grid_constant__ LocalParams P, int64_t batch, const int
                     const double v = __shfl_sync(0xffffffffu, sol.inc, r);
                     const unsigned long long bm = __shfl_sync(0xffffffffu, (unsigned long long)sol.best_modes, r);
                     const int nn = __shfl_sync(0xffffffffu, sol.nodes, r), ii = __shfl_sync(0xffffffffu, sol.iters, r);
-                    const int tr = __shfl_sync(0xffffffffu, (int)sol.trouble, r);
+                    // the owner's status is the worst of its own and its adopters' (time-out > node limit > numeric)
+                    const int tr = __shfl_sync(0xffffffffu, (int)sol.trouble | ((int)sol.timeout << 1) | ((int)sol.limit << 2), r);
                     __syncwarp();
                     if (lane == o) {
                         --pending;
                         sol.nodes += nn; sol.iters += ii;
-                        if (tr) sol.trouble = true;
+                        if (tr & 1) sol.trouble = true;
+                        if (tr & 2) sol.timeout = true;
+                        if (tr & 4) sol.limit = true;
                         if (v < sol.inc) {
                             sol.inc = v; sol.best_modes = bm;
                             const double* src = scratch + ((size_t)blockIdx.x * 32 + r) * N;
@@ -208,6 +211,7 @@ flat_miqp_kernel(const __grid_constant__ LocalParams P, int64_t batch, const int
             bool start = false, adopting = false;
             int a_l = 0, a_c = 0, a_owner = lane;
             unsigned long long a_modes = 0;
+            long long a_t0 = 0;
             double a_inc = 0.0;
             const unsigned need = __ballot_sync(0xffffffffu, !have);
             if (need && !drained) {
@@ -236,6 +240,7 @@ flat_miqp_kernel(const __grid_constant__ LocalParams P, int64_t batch, const int
                     const long long di = __shfl_sync(0xffffffffu, (long long)i, d);
                     const unsigned long long dm = __shfl_sync(0xffffffffu, (unsigned long long)sol.modes_pk, d);
                     const double dinc = __shfl_sync(0xffffffffu, sol.inc, d);
+                    const long long dt0 = __shfl_sync(0xffffffffu, cold.t_start, d);     // the problem's clock
                     int m = __popc((unsigned)dcb) - (dtot == __popc((unsigned)dcb) ? 1 : 0);   // the donor keeps work
                     if (m > __popc(idle)) m = __popc(idle);
                     if (m <= 0) continue;
@@ -244,7 +249,7 @@ flat_miqp_kernel(const __grid_constant__ LocalParams P, int64_t batch, const int
                     if (me_idle && rk < m) {
                         int bits = dcb;
                         for (int t = 0; t < rk; ++t) bits &= bits - 1;
-                        a_c = __ffs(bits) - 1; a_l = dl; a_modes = dm; a_inc = dinc; a_owner = d;
+                        a_c = __ffs(bits) - 1; a_l = dl; a_modes = dm; a_inc = dinc; a_owner = d; a_t0 = dt0;
                         i = di; start = true; adopting = true;
                     }
                     if (lane == d) {
@@ -260,7 +265,10 @@ flat_miqp_kernel(const __grid_constant__ LocalParams P, int64_t batch, const int
                 sol.setup(smem + lane, &P, flags[i], mass[i], x0 + 2 * i, xf ? xf + S * i : nullptr,
                           xb ? xb + S * i : nullptr, xl ? xl + S * i : nullptr,
                           adopting ? my_scratch : x + S * i + (N + 2), &cold);
-                if (STEAL && adopting) sol.adopt_prefix(a_modes, a_l, a_c, a_inc);
+                if (STEAL && adopting) {
+                    sol.adopt_prefix(a_modes, a_l, a_c, a_inc);
+                    cold.t_start = a_t0;       // one problem, one budget: an adopted branch keeps the owner's clock
+                }
                 else if (HINTS && P.hint) sol.apply_hint(P.hint + (size_t)N * i);
                 have = true; thief = adopting; owner = a_owner;
             }

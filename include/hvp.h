@@ -112,7 +112,9 @@ typedef struct {
     /* Solver options (SURVEY.md 8b; Gurobi parameters of mpcs/mpc_gear.py:182-186, Q12).  mip_gap: relative gap at
      * which a node is pruned (Gurobi MIPGap, default there 1e-4); 0 = proven optimal.  time_limit_ms: budget per
      * problem, measured on the device from the moment the problem is picked up; when it runs out the incumbent is
-     * returned with status HVP_TIME_LIMIT (9); 0 = none. */
+     * returned with status HVP_TIME_LIMIT (9); 0 = none.  Sub-trees that other lanes or warps search for the problem
+     * (the split of small batches, adoption in the tail of a flat launch) run on the same budget, and a time-out in
+     * any of them makes the problem's status HVP_TIME_LIMIT. */
     double mip_gap;
     double time_limit_ms;
     /* Optional incumbent hint for hvp_local_miqp_dev: DEVICE pointer to [batch][N] int32 region sequences (the codes

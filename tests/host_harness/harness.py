@@ -12,7 +12,7 @@ _ip = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
 
 
 def build(force=False):
-    srcs = [os.path.join(_HERE, "harness.cpp"),
+    srcs = [os.path.join(_HERE, "harness.cpp"), os.path.join(_HERE, "scalar_solver.h"),
             os.path.join(_HERE, "../../hybrid_vehicle_platoon_b200/csrc/miqp_core.cuh"),
             os.path.join(_HERE, "../../hybrid_vehicle_platoon_b200/csrc/vehicle_model.h"),
             os.path.join(_HERE, "../../hybrid_vehicle_platoon_b200/csrc/coop_core.cuh"),
@@ -27,15 +27,17 @@ def build(force=False):
 def local_miqp(N, flags, mass, x0, xf, xb, xl, d0=50.0, t0=0.0, tight=0.0, max_nodes=0, coop=False, flat=False):
     L = C.CDLL(build())
     fn = L.hvh_flat_miqp_batch if flat else (L.hvh_coop_miqp_batch if coop else L.hvh_local_miqp_batch)
+    # references may be None (NULL): legal for the roles that do not read them
     fn.argtypes = [C.c_int, C.c_int, _ip, C.c_double, C.c_double, C.c_double,
-                                       C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _ip, _dp, _ip,
+                                       C.c_int, _dp, _dp, C.c_void_p, C.c_void_p, C.c_void_p, _dp, _dp, _ip, _dp, _ip,
                                        _ip, _ip]
     B = x0.shape[0]
     c = lambda a, t=np.float64: np.ascontiguousarray(a, dtype=t)
+    refs = [None if a is None else c(a) for a in (xf, xb, xl)]
+    ptr = lambda a: None if a is None else a.ctypes.data
     u = np.zeros((B, N)); x = np.zeros((B, 2, N + 1)); modes = np.zeros((B, N), np.int32)
     obj = np.zeros(B); st = np.zeros(B, np.int32); nodes = np.zeros(B, np.int32); it = np.zeros(B, np.int32)
-    fn(B, N, c(flags, np.int32), d0, t0, tight, max_nodes, c(mass), c(x0), c(xf),
-                           c(xb), c(xl), u, x, modes, obj, st, nodes, it)
+    fn(B, N, c(flags, np.int32), d0, t0, tight, max_nodes, c(mass), c(x0), *map(ptr, refs), u, x, modes, obj, st, nodes, it)
     return dict(u=u, x=x, modes=modes, obj=obj, status=st, nodes=nodes, qp_iters=it)
 
 

@@ -47,6 +47,7 @@ struct LocalSolver {
     double hw1, hw2, hd;               // tracking Hessian closed form
     double ct;                         // tracking constant (incl. k = 0,1 slack penalties)
     bool has_sf, has_sb;
+    bool notrack;                               // no reference term (setup)
     int L;                             // stages 0..L-1 have fixed regions
     uint64_t modes_pk;                 // 3 bits per stage
     uint64_t act_lo, act_hi;           // active constraint ids (8 bits each: t*12 + j)
@@ -97,6 +98,7 @@ struct LocalSolver {
         hw1 = 2.0 * wp * nterm;
         hw2 = 2.0 * wp * (tf ? t0 : 0.0);
         hd = 2.0 * wp * (tf ? t0 * t0 : 0.0) + 2.0 * wvv * nterm;
+        notrack = nterm < 0.5;     // no reference term: the Hessian is singular until every stage is fixed
         for (int j = 0; j < N; ++j) w(LY::O_GT, j) = 0.0;
         ct = 0.0;
         // rho_k = pc - Pk (k>=1);  g[j] = 2wp*(sum_{k>j+1} rho_k + tau*rho_{j+1}) - 2wv*V_{j+1}
@@ -481,6 +483,15 @@ struct LocalSolver {
             }
             // p_1 = pc is a constant: its state rows are a feasibility check
             if (pc > P->pmax + eps || pc < P->pmin - eps) continue;
+            if (notrack && L < N) {                         // only leaves are solved (enumeration, as the oracle)
+                ++lev;
+                w(LY::O_XSTAR, lev) = w(LY::O_XSTAR, lev - 1);
+                int cn = 0;
+                for (int c = 0; c < NREG; ++c)
+                    if (P->edge[c] <= w(LY::O_RHI, lev) && P->edge[c + 1] >= w(LY::O_RLO, lev)) cn |= (1 << c);
+                HVP_CAND_SET(lev, cn);
+                continue;
+            }
             double obj;
             const int st = solve_node(&obj);
             ++R.nodes;

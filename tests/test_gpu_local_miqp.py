@@ -196,10 +196,14 @@ def test_modes_hint_never_changes_the_optimum(hvp_ctx):
 def test_more_streams_than_launch_slots(hvp_ctx):
     """The library keeps the launch state of the per-vehicle kernel (work counter, adoption scratch) per STREAM, for 64
     streams; a caller that keeps creating streams takes over the least recently used slot whose last launch has finished.
-    90 fresh streams one after the other, then 8 of them in flight at once: every launch returns the first one's answers
-    (objective to round-off -- adoption makes the order of incumbents timing-dependent -- statuses exactly)."""
+    90 distinct streams one after the other, then 8 of them in flight at once: every launch returns the first one's
+    answers (objective to round-off -- adoption makes the order of incumbents timing-dependent -- statuses exactly).
+    torch.cuda.Stream() hands out a pool of 32 streams round robin, so the streams are created with cudaStreamCreate."""
+    import ctypes
     import torch
     from hybrid_vehicle_platoon_b200 import api
+    torch.cuda.init()
+    cudart = ctypes.CDLL("libcudart.so.12")
     rng = np.random.default_rng(33)
     N, n, S = 6, 10, 1024                                   # 10 240 problems: the flat kernel
     c = platoon_local_problems(rng, S, n, N, stress=True)
@@ -226,14 +230,23 @@ def test_more_streams_than_launch_slots(hvp_ctx):
         assert torch.equal(o["st"], base["st"])
         assert torch.allclose(o["ob"][ok], base["ob"][ok], rtol=1e-9, atol=0)
 
-    keep = []
-    for _ in range(90):
-        s = torch.cuda.Stream(device=dev)
-        keep.append(s)
-        o = launch(s)
-        s.synchronize()
-        same(o)
-    outs = [launch(s) for s in keep[-8:]]                   # eight launches in flight, each on a stream of its own
-    torch.cuda.synchronize()
-    for o in outs:
-        same(o)
+    handles, keep = [], []
+    try:
+        for _ in range(90):
+            h = ctypes.c_void_p()
+            assert cudart.cudaStreamCreate(ctypes.byref(h)) == 0
+            handles.append(h)
+            s = torch.cuda.ExternalStream(h.value, device=dev)
+            keep.append(s)
+            o = launch(s)
+            s.synchronize()
+            same(o)
+        assert len({s.cuda_stream for s in keep}) > 64          # more streams than launch slots: the takeover runs
+        outs = [launch(s) for s in keep[-8:]]                   # eight launches in flight, each on a stream of its own
+        torch.cuda.synchronize()
+        for o in outs:
+            same(o)
+    finally:
+        torch.cuda.synchronize()
+        for h in handles:
+            cudart.cudaStreamDestroy(h)
